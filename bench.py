@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # the CUDA engine
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's output
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): 64 independent
 dspu::Convolver instances per GPU, 480 000-tap (10 s @ 48 kHz) synthetic exponentially-decaying
@@ -40,6 +41,7 @@ BYTES_PER_INSTANCE_FRAME = 16 * F * BINS + 24 * F
 METRIC = "Convolver output samples/s (64ch x 10s IR, 1024-sample blocks)"
 UNIT = "samples/s"
 FALLBACK_HBM_GBS = 6650.0
+DUMP_ROWS, DUMP_BYTES = 16, 60_000_000
 
 
 def hbm_peak():
@@ -118,6 +120,24 @@ def cpu_reference_rate(threads, blocks, warm=4):
     impl = "reference" if kind == "reference" else "oracle"
     rate, sec = bindings.cpu_bench(impl, threads, TAPS, RANK, BLOCK, warm, blocks, threads)
     return rate, sec, kind
+
+
+def dump_outputs(path, dst):
+    """Saves what the last timed step returned to its caller, ``dst`` = [64 instances][frames * 1024]
+    float32, as ``path/convolver_dst.npy``: the rows of a fixed, seeded choice of 16 instances, in
+    instance order, every sample of the step (a seeded, sorted choice of columns when a longer step
+    would exceed DUMP_BYTES).  The inputs are seeded too, so two builds can be compared sample for sample."""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(0)
+    rows = np.sort(rng.choice(dst.shape[0], DUMP_ROWS, replace=False))
+    out = dst[torch.as_tensor(rows, device=dst.device)]
+    limit = DUMP_BYTES // (4 * DUMP_ROWS)
+    if out.shape[1] > limit:
+        cols = np.sort(rng.choice(out.shape[1], limit, replace=False))
+        out = out[:, torch.as_tensor(cols, device=dst.device)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "convolver_dst.npy"), out.cpu().numpy())
 
 
 def run_reference(args, rank, world):
@@ -392,7 +412,12 @@ def main():
     ap.add_argument("--extras-timeout", type=int, default=420)
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the extra multi-GPU shapes (cfg3 strong scaling, cfg5 partition split)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step (rank 0, a seeded sample of 16 instances) "
+                         "to DIR/convolver_dst.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -476,6 +501,8 @@ def main():
         step_ms = sorted(edges[i].elapsed_time(edges[i + 1]) for i in range(args.steps))
         clocks = sampler.stop() if rank == 0 else None
         stats = batch.stats()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dst)
 
         # ---- roofline pass: per-launch duration of k_mac, CUDA events on the launching stream ---
         batch.set_profiling(True)

@@ -58,8 +58,9 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 def build(verbose=False):
     """Compile csrc/engine.cu for sm_100a into libb200conv.so (in-tree)."""
     src = os.path.join(_HERE, "csrc", "engine.cu")
-    deps = [src, os.path.join(_HERE, "csrc", "kernels.cuh"), os.path.join(_HERE, "csrc", "equalizer.cuh"),
-            os.path.join(_ROOT, "include", "b200conv.h")]
+    deps = [src, os.path.join(_ROOT, "include", "b200conv.h")] + [
+        os.path.join(_HERE, "csrc", h) for h in ("kernels.cuh", "equalizer.cuh", "spectral.cuh", "spectral_host.cuh",
+                                                  "splitter.cuh")]
     if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
     cmd = ["nvcc"] + NVCC_FLAGS + ["-I", os.path.join(_ROOT, "include"), "-o", LIB_PATH, src]

@@ -37,3 +37,12 @@ class ModelSpectralProcessor:
             self.off += n
             pos += n
         return out
+
+    def remaining(self):
+        """Samples until the next transform (SpectralProcessor::remaining, :241-245)."""
+        return self.F - self.off
+
+    def reset(self):
+        """SpectralProcessor::reset (:247-257): buffers cleared, offset kept."""
+        self.inb[:] = 0.0
+        self.outb[:] = 0.0

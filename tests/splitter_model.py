@@ -28,6 +28,9 @@ class ModelSpectralSplitter:
         self.cur = [np.zeros(self.F) for _ in range(handlers)]      # what the sink sees during the current hop
         self.fill = self.f0                 # nFrameSize
 
+    def latency(self):
+        return 2 * self.F
+
     def bind(self, handler, hook):
         self.hooks[handler] = hook
         self.tail[handler] = np.zeros(self.F)

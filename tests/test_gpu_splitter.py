@@ -1,10 +1,13 @@
 """Scope-table row f4, second sibling, on the GPU: the batched SpectralSplitter (b200conv_ss_*)
-against the reference's own class (SpectralSplitter.cpp compiled verbatim into oracle/_ref, host
-callbacks in oracle/ref_wrap_splitter.cpp) and the float64 model (tests/splitter_model.py)."""
+against the outputs of the reference's own class frozen in tests/golden/spectral_golden.npz, the
+float64 model of the reference class (tests/splitter_model.py, held to the frozen outputs by
+tests/test_oracle_spectral_golden.py) and, where oracle/_ref has been built, the reference class
+itself (SpectralSplitter.cpp compiled verbatim, host callbacks in oracle/ref_wrap_splitter.cpp)."""
 import numpy as np
 import pytest
 
 import splitter_model
+import spectral_cases as cases
 import synth
 from oracle.bindings import CpuSpectralSplitter
 
@@ -20,14 +23,6 @@ def pkg():
     return p
 
 
-def _tables(rank, seed):
-    N = 1 << rank
-    rng = np.random.Generator(np.random.PCG64(seed))
-    gain = rng.uniform(0.2, 1.5, N).astype(np.float32)                          # NOT symmetric on purpose
-    H = (rng.uniform(-1, 1, N) + 1j * rng.uniform(-1, 1, N)).astype(np.complex64)      # NOT conjugate-symmetric
-    return gain, H
-
-
 def _close(got, want):
     return np.max(np.abs(got.astype(np.float64) - want)) <= TOL * max(1.0, np.max(np.abs(want)))
 
@@ -36,10 +31,8 @@ def _close(got, want):
                                              (13, 11, 10000), (14, 0, 8192), (14, 9, 3000)])
 def test_batch_against_the_reference_class(pkg, rank, chunk, step):
     """Instances with different phases and handler sets (real gains / complex table / sink only /
-    unbound) in one batch, arbitrary call sizes: every band of every instance against the reference
-    class."""
-    if not CpuSpectralSplitter.available():
-        pytest.skip("oracle/_ref has not been built")
+    unbound) in one batch, arbitrary call sizes: every band of every instance against the model of
+    the reference class."""
     N = 1 << rank
     n = 5 * N + 123
     H4 = 4
@@ -51,35 +44,60 @@ def test_batch_against_the_reference_class(pkg, rank, chunk, step):
         ss.set_chunk_rank(chunk)
     refs = []
     for c, (kinds, ph) in enumerate(setups):
-        ref = CpuSpectralSplitter(14, H4)
-        ref.set_rank(rank)
-        if chunk:
-            ref.set_chunk_rank(chunk)
-        ref.set_phase(ph)
+        ref = splitter_model.ModelSpectralSplitter(rank, H4, chunk, ph)
         ss.set_phase(c, ph)
         for h, kind in enumerate(kinds):
-            gain, H = _tables(rank, 100 * rank + 10 * c + h)
+            gain, H = cases.tables(rank, 100 * rank + 10 * c + h)
             if kind == 1:
-                ref.bind_complex(h, H)
+                ref.bind(h, lambda X, H=H: X * H.astype(np.complex128))
                 ss.bind_complex(c, h, H)
             elif kind == 2:
-                ref.bind_gain(h, gain)
+                ref.bind(h, lambda X, gain=gain: X * gain.astype(np.float64))
                 ss.bind_gain(c, h, gain)
             elif kind == 3:
-                ref.bind_sink(h)
+                ref.bind(h, "copy")
                 ss.bind_sink(c, h)
-        assert ss.bindings(c) == ref.bindings()
+        assert ss.bindings(c) == sum(kind != 0 for kind in kinds)
         refs.append(ref)
     got = np.concatenate([ss.process(x[:, i:i + step]) for i in range(0, n, step)], axis=2)
+    assert ss.latency() == refs[0].latency() and 1 << ss.chunk_rank() == refs[0].latency()
     for c, (kinds, ph) in enumerate(setups):
-        want = refs[c].run(x[c], step)
-        if any(kinds):                      # (the reference commits its settings in process())
-            assert ss.latency() == refs[c].latency() and ss.chunk_rank() == refs[c].chunk_rank()
+        want = refs[c].process(x[c])
         for h, kind in enumerate(kinds):
             if kind == 0:
                 assert np.all(got[h, c] == 0.0)
             else:
-                assert _close(got[h, c], want[h].astype(np.float64)), (c, h, kind)
+                assert _close(got[h, c], want[h]), (c, h, kind)
+    ss.close()
+
+
+@pytest.mark.parametrize("name", [c[0] for c in cases.SS_CASES])
+def test_frozen_reference_outputs(pkg, name):
+    """The cases of tests/golden/spectral_golden.npz: what the reference class itself produced."""
+    g = np.load(cases.GOLDEN)
+    rank, chunk, phase, step, latency, seed, n = g[name + ".meta"]
+    rank, chunk, step, seed, n = int(rank), int(chunk), int(step), int(seed), int(n)
+    kinds = [int(k) for k in g[name + ".kinds"]]
+    src = synth.noise(seed, n)
+    ss = pkg.SpectralSplitterBatch(1, 13, len(kinds), device=0)
+    ss.set_rank(rank)
+    if chunk:
+        ss.set_chunk_rank(chunk)
+    ss.set_phase(0, float(phase))
+    for h, kind in enumerate(kinds):
+        gain, H = cases.tables(rank, 10 * seed + h)
+        if kind == 1:
+            ss.bind_complex(0, h, H)
+        elif kind == 2:
+            ss.bind_gain(0, h, gain)
+        elif kind == 3:
+            ss.bind_sink(0, h)
+    got = np.concatenate([ss.process(src[None, i:i + step])[:, 0] for i in range(0, n, step)], axis=1)
+    want = g[name + ".dst"].astype(np.float64)
+    bound = [h for h, kind in enumerate(kinds) if kind != 0]
+    assert _close(got[bound], want)
+    assert np.all(got[[h for h, kind in enumerate(kinds) if kind == 0]] == 0.0)
+    assert ss.latency() == int(latency)
     ss.close()
 
 
@@ -122,7 +140,7 @@ def test_settings_rebinding_device_api_and_errors(pkg):
     with pytest.raises(Exception):
         pkg.SpectralSplitterBatch(1, 15, 1, device=0)   # ranks 7..14
     ss.set_rank(rank)
-    gain, H = _tables(rank, 9)
+    gain, H = cases.tables(rank, 9)
     for c in range(inst):
         ss.bind_gain(c, 0, gain)
         ss.bind_complex(c, 1, H)

@@ -1,27 +1,21 @@
 """Scope-table row f4: outputs of the reference's own SpectralProcessor / SpectralSplitter frozen in
-tests/golden/spectral_golden.npz (tests/golden/make_golden_spectral.py).  The verbatim build must
-reproduce them bit for bit (it does not depend on the machine: scalar restated kernels, no FMA
-contraction in the schedulers), and the independent float64 models must agree with them.  CPU only."""
-import importlib.util
-import os
-
+tests/golden/spectral_golden.npz (tests/golden/make_golden_spectral.py; the cases are listed in
+tests/spectral_cases.py).  The verbatim build must reproduce them bit for bit (it does not depend on
+the machine: scalar restated kernels, no FMA contraction in the schedulers), and the independent
+float64 models must agree with them.  CPU only."""
 import numpy as np
 import pytest
 
+import spectral_cases as cases
 import spectral_model
 import splitter_model
 import synth
 from oracle.bindings import CpuSpectralProcessor, CpuSpectralSplitter
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-spec = importlib.util.spec_from_file_location("make_golden_spectral", os.path.join(HERE, "golden", "make_golden_spectral.py"))
-gen = importlib.util.module_from_spec(spec)
-spec.loader.exec_module(gen)
-
 
 @pytest.fixture(scope="module")
 def golden():
-    return np.load(os.path.join(HERE, "golden", "spectral_golden.npz"))
+    return np.load(cases.GOLDEN)
 
 
 def _hook(kind, gain, H):
@@ -33,11 +27,11 @@ def _hook(kind, gain, H):
 
 
 def test_spectral_processor_cases(golden):
-    for name, *_ in gen.SP_CASES:
+    for name, *_ in cases.SP_CASES:
         rank, phase, step, kind, latency, seed, n = golden[name + ".meta"]
         rank, step, kind, seed, n = int(rank), int(step), int(kind), int(seed), int(n)
         src = synth.noise(seed, n)
-        gain, H = gen.tables(rank, seed)
+        gain, H = cases.tables(rank, seed)
         want = golden[name + ".dst"]
         model = spectral_model.ModelSpectralProcessor(rank, float(phase), _hook(kind, gain, H)).process(src)
         assert np.max(np.abs(model - want)) <= 2e-5 * max(1.0, np.max(np.abs(want))), name
@@ -54,7 +48,7 @@ def test_spectral_processor_cases(golden):
 
 
 def test_spectral_splitter_cases(golden):
-    for name, *_ in gen.SS_CASES:
+    for name, *_ in cases.SS_CASES:
         rank, chunk, phase, step, latency, seed, n = golden[name + ".meta"]
         rank, chunk, step, seed, n = int(rank), int(chunk), int(step), int(seed), int(n)
         kinds = [int(k) for k in golden[name + ".kinds"]]
@@ -69,7 +63,7 @@ def test_spectral_splitter_cases(golden):
                 ref.set_chunk_rank(chunk)
             ref.set_phase(float(phase))
         for h, kind in enumerate(kinds):
-            gain, H = gen.tables(rank, 10 * seed + h)
+            gain, H = cases.tables(rank, 10 * seed + h)
             if kind == 3:
                 m.bind(h, "copy")
             elif kind != 0:
