@@ -460,6 +460,57 @@ size_t  b200conv_ss_latency(const b200conv_ss_t *s);
 size_t  b200conv_ss_instances(const b200conv_ss_t *s);
 size_t  b200conv_ss_handlers(const b200conv_ss_t *s);
 
+/* ---- matrix convolver: many inputs x many outputs through routed impulse responses ----------
+ * `inputs` I and `outputs` O at one rank, and a list of routes (input i, output o, impulse response h).
+ * Every call produces, with zero latency, for every output
+ *     y_o[n] = sum over the routes r with output(r) = o of  sum_k h_r[k] x_input(r)[n - k]
+ * over every sample since the last b200conv_mx_set_routes / b200conv_mx_clear.  The arithmetic plan is
+ * the convolver's (uniform partitions of F = 2^(rank-1) samples, folded overlap, a frequency-domain
+ * delay line); what is shared is ONE input-spectrum ring per input, whatever the number of routes that
+ * read it, and ONE inverse transform per output, whatever the number of routes summed into it.  A
+ * true-stereo reverb (2 x 2, 4 routes), an ambisonic room response (1 x 16) or a binaural decoder
+ * (16 x 2, each ear a sum of 16 convolutions) is one object.
+ *
+ *   b200conv_mx_create          ranks 8..16 (B200CONV_ERR_ARG otherwise), 1..4096 inputs and outputs;
+ *                               until the first set_routes every output is zeros
+ *   b200conv_mx_set_routes      replaces the whole routing: route r reads input[r], adds into output[r]
+ *                               through ir[r][0 .. length[r]) (HOST pointers, borrowed for the call only).
+ *                               length[r] >= 1, indices in range, each (input, output) pair at most once,
+ *                               else B200CONV_ERR_ARG; count == 0 is valid (every output is zeros).  All
+ *                               input history is discarded.  On B200CONV_ERR_ARG / _ERR_NOMEM nothing
+ *                               changes (the old routes and history stay).  Ordered after every call
+ *                               already enqueued on the object; synchronous
+ *   b200conv_mx_clear           discards the input history, keeps the routes
+ *   b200conv_mx_process_device  src: DEVICE matrix [inputs][src_stride], dst: DEVICE matrix
+ *                               [outputs][dst_stride] floats; count must be a multiple of F (0 = no-op;
+ *                               anything else returns B200CONV_ERR_ARG and changes nothing).  Outputs with
+ *                               no route get zeros; dst == src with equal strides is allowed.  Enqueued on
+ *                               `stream` (a cudaStream_t; NULL = the object's own stream) without host
+ *                               synchronisation; all calls on one object must be ordered on one stream (or
+ *                               be separated by b200conv_mx_sync)
+ *   b200conv_mx_process_planar  the same on HOST matrices; synchronous
+ *   b200conv_mx_sync            waits for everything the object has enqueued
+ *   b200conv_mx_frame_size      F: the call-size granule
+ *   b200conv_mx_routes          routes of the current routing */
+typedef struct b200conv_mx b200conv_mx_t;
+
+int     b200conv_mx_create(b200conv_mx_t **out, int device, size_t inputs, size_t outputs, size_t rank);
+void    b200conv_mx_free(b200conv_mx_t *m);
+int     b200conv_mx_set_routes(b200conv_mx_t *m, size_t count, const size_t *input, const size_t *output,
+                               const float *const *ir, const size_t *length);
+int     b200conv_mx_clear(b200conv_mx_t *m);
+int     b200conv_mx_process_device(b200conv_mx_t *m, float *dst, size_t dst_stride, const float *src,
+                                   size_t src_stride, size_t count, void *stream);
+int     b200conv_mx_process_planar(b200conv_mx_t *m, float *dst, size_t dst_stride, const float *src,
+                                   size_t src_stride, size_t count);
+int     b200conv_mx_sync(b200conv_mx_t *m);
+void   *b200conv_mx_stream(b200conv_mx_t *m);
+size_t  b200conv_mx_inputs(const b200conv_mx_t *m);
+size_t  b200conv_mx_outputs(const b200conv_mx_t *m);
+size_t  b200conv_mx_rank(const b200conv_mx_t *m);
+size_t  b200conv_mx_frame_size(const b200conv_mx_t *m);
+size_t  b200conv_mx_routes(const b200conv_mx_t *m);
+
 /* ---- misc -------------------------------------------------------------------------------- */
 
 const char *b200conv_last_error(void);      /* thread-local text of the last failure */

@@ -60,7 +60,7 @@ def build(verbose=False):
     src = os.path.join(_HERE, "csrc", "engine.cu")
     deps = [src, os.path.join(_ROOT, "include", "b200conv.h")] + [
         os.path.join(_HERE, "csrc", h) for h in ("kernels.cuh", "equalizer.cuh", "spectral.cuh", "spectral_host.cuh",
-                                                  "splitter.cuh")]
+                                                  "splitter.cuh", "matrix.cuh", "matrix_host.cuh")]
     if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
     cmd = ["nvcc"] + NVCC_FLAGS + ["-I", os.path.join(_ROOT, "include"), "-o", LIB_PATH, src]
@@ -161,6 +161,20 @@ _SIGNATURES = {
     "b200conv_ss_latency": (_SZ, [_VP]),
     "b200conv_ss_instances": (_SZ, [_VP]),
     "b200conv_ss_handlers": (_SZ, [_VP]),
+    "b200conv_mx_create": (ctypes.c_int, [ctypes.POINTER(_VP), ctypes.c_int, _SZ, _SZ, _SZ]),
+    "b200conv_mx_free": (None, [_VP]),
+    "b200conv_mx_set_routes": (ctypes.c_int, [_VP, _SZ, ctypes.POINTER(_SZ), ctypes.POINTER(_SZ), ctypes.POINTER(_FP),
+                                              ctypes.POINTER(_SZ)]),
+    "b200conv_mx_clear": (ctypes.c_int, [_VP]),
+    "b200conv_mx_process_device": (ctypes.c_int, [_VP, _VP, _SZ, _VP, _SZ, _SZ, _VP]),
+    "b200conv_mx_process_planar": (ctypes.c_int, [_VP, _VP, _SZ, _VP, _SZ, _SZ]),
+    "b200conv_mx_sync": (ctypes.c_int, [_VP]),
+    "b200conv_mx_stream": (_VP, [_VP]),
+    "b200conv_mx_inputs": (_SZ, [_VP]),
+    "b200conv_mx_outputs": (_SZ, [_VP]),
+    "b200conv_mx_rank": (_SZ, [_VP]),
+    "b200conv_mx_frame_size": (_SZ, [_VP]),
+    "b200conv_mx_routes": (_SZ, [_VP]),
     "b200conv_last_error": (ctypes.c_char_p, []),
     "b200conv_version": (ctypes.c_char_p, []),
 }
@@ -682,3 +696,67 @@ class SpectralSplitterBatch:
 
     def stream(self):
         return lib().b200conv_ss_stream(self._h)
+
+
+class MatrixConvolver:
+    """``inputs`` x ``outputs`` matrix of routed convolutions on one GPU (``b200conv_mx_*``): output ``o``
+    is the sum, over the routes ``(i, o, ir)``, of input ``i`` convolved with ``ir``.  One spectrum ring
+    per input and one inverse transform per output, whatever the number of routes.  Calls must bring
+    whole frames (a multiple of ``frame_size()`` samples)."""
+
+    def __init__(self, inputs, outputs, rank, device=-1):
+        self._h = _VP()
+        _check(lib().b200conv_mx_create(ctypes.byref(self._h), device, inputs, outputs, rank))
+        self.inputs = inputs
+        self.outputs = outputs
+        self.rank = rank
+
+    def close(self):
+        if self._h:
+            lib().b200conv_mx_free(self._h)
+            self._h = _VP()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def set_routes(self, routes):
+        """``routes``: ``[(input, output, ir), ...]``; replaces the routing and discards the history."""
+        routes = list(routes)
+        n = len(routes)
+        irs = [np.ascontiguousarray(h, dtype=np.float32) for _, _, h in routes]
+        _check(lib().b200conv_mx_set_routes(self._h, n, (_SZ * n)(*[int(r[0]) for r in routes]),
+                                            (_SZ * n)(*[int(r[1]) for r in routes]),
+                                            (_FP * n)(*[_ptr(h) for h in irs]), (_SZ * n)(*[h.size for h in irs])))
+
+    def clear(self):
+        _check(lib().b200conv_mx_clear(self._h))
+
+    def process(self, src):
+        """src: [inputs][n] float32 (host) -> [outputs][n] (synchronous)."""
+        src = np.ascontiguousarray(src, dtype=np.float32)
+        if src.ndim != 2 or src.shape[0] != self.inputs:
+            raise ValueError("expected [inputs][samples]")
+        n = src.shape[1]
+        out = np.empty((self.outputs, n), dtype=np.float32)
+        _check(lib().b200conv_mx_process_planar(self._h, out.ctypes.data, n, src.ctypes.data, n, n))
+        return out
+
+    def process_device(self, dst_ptr, dst_stride, src_ptr, src_stride, n, stream=None):
+        """Device pointers (ints): ``src`` [inputs][src_stride], ``dst`` [outputs][dst_stride] floats;
+        stream-ordered (``stream`` None = the object's own stream)."""
+        _check(lib().b200conv_mx_process_device(self._h, dst_ptr, dst_stride, src_ptr, src_stride, n, stream))
+
+    def sync(self):
+        _check(lib().b200conv_mx_sync(self._h))
+
+    def stream(self):
+        return lib().b200conv_mx_stream(self._h)
+
+    def frame_size(self):
+        return int(lib().b200conv_mx_frame_size(self._h))
+
+    def routes(self):
+        return int(lib().b200conv_mx_routes(self._h))

@@ -18,6 +18,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <algorithm>
 #include <new>
 #include <string>
 #include <thread>
@@ -3187,6 +3188,8 @@ extern "C" int b200conv_chirp_linear_convolutions(int device, float *result, siz
 #include "spectral.cuh"
 #include "spectral_host.cuh"
 #include "splitter.cuh"
+#include "matrix.cuh"
+#include "matrix_host.cuh"
 
 #ifdef B200CONV_TIMING
 /* developer instrumentation: copies the per-CTA timestamps of the last k_frame launch */
