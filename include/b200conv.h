@@ -81,6 +81,8 @@ typedef struct b200conv_stats
     uint64_t d2h_bytes;         /* bytes copied device -> host by b200conv_process                  */
     uint64_t mac_launches;      /* launches of the partition MAC kernel                             */
     uint64_t mac_algo_bytes;    /* algorithmic bytes of those launches (DESIGN.md: 16*F*bins + 24*F per instance-frame) */
+    uint64_t mac_stream_bytes;  /* bytes those launches actually stream: less than mac_algo_bytes when one-frame calls
+                                   run with lookahead (option "lookahead"), each IR spectrum row read once per K blocks */
 } b200conv_stats_t;
 
 /* ---- lifetime -------------------------------------------------------------------------- */
@@ -232,6 +234,12 @@ void   *b200conv_stream(b200conv_batch_t *h);
  *                 inverse transform of block t and streams under it and under the transform of block
  *                 t + 1; partition 0 is added by that block's inverse transform.  Rows computed ahead
  *                 for a block that then arrives differently are simply not used; 0 = off
+ *   "lookahead"   ranks 8..13, streams of one-frame calls in uniform mode: the launches of a group of
+ *                 K blocks also sum, each over one bin slice, the partitions q >= 2K of the next
+ *                 group's blocks (they need frames that are already in the ring), so each IR spectrum
+ *                 row is streamed once per K blocks.  -1 (default) = automatic (bandwidth-bound
+ *                 batches only); 0 = off; 2, 4, 8 = that K.  Results differ from "off" only in the
+ *                 order of the partition sum
  *   "mac_tile"    developer knob, ranks 14..16, process-wide: bins per k_mac CTA (0 = 1024, 512, 256)
  *   "zero_copy"   1 (default) = b200conv_process_planar lets the kernels read / write page-locked
  *                 host matrices directly (no staging copies); 0 = always stage */

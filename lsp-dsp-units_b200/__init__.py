@@ -42,7 +42,7 @@ class Dump(ctypes.Structure):
 
 class Stats(ctypes.Structure):
     _fields_ = [(n, ctypes.c_uint64) for n in ("launches", "frames", "h2d_bytes", "d2h_bytes",
-                                               "mac_launches", "mac_algo_bytes")]
+                                               "mac_launches", "mac_algo_bytes", "mac_stream_bytes")]
 
 
 class B200ConvError(RuntimeError):

@@ -658,6 +658,9 @@ static_assert(FRAME_CHAIN_MAX < RING_SPARE, "k_frame launches in flight must fit
 static const uint64_t EARLY_MAX_BYTES = 450000000ull;  /* launches that stream more than this per block (~70 us) keep the
                                                            in-kernel wait: they hide the chain anyway, and spare themselves
                                                            the serialised launch every FRAME_CHAIN_MAX blocks */
+static const uint64_t LA_MIN_BYTES = 64000000ull;      /* k_frame lookahead: only launches that stream at least this per
+                                                           block (bandwidth-bound); shorter ones are latency-bound and
+                                                           would only pay for the extra T rows in their tail */
 static const size_t PART_MAX   = 1024;                  /* samples one P1 / P2 segment of a fused step answers */
 
 struct b200conv_batch
@@ -726,6 +729,17 @@ struct b200conv_batch
     uint64_t                ahead_t     = 0;
     uint32_t                ahead_splits = 0;
     uint32_t               *h_error     = nullptr;  /* page-locked, device-mapped: a bounded in-kernel wait gave up */
+    /* k_frame lookahead for one-frame calls (kernels.cuh, LA_BUFS) */
+    int                     opt_lookahead = -1;     /* -1 automatic, 0 off, 2 / 4 / 8 = that group size K */
+    float2                 *la_T        = nullptr;  /* [LA_BUFS][jobs][K][splits][M] */
+    size_t                  la_T_bytes  = 0;
+    uint32_t               *d_la_cnt    = nullptr;  /* [2][LA_BUFS][instances]: producer CTAs, consumer tails */
+    bool                    la_live     = false;    /* the last launch of this batch was a lookahead k_frame (la_* below) */
+    uint32_t                la_K        = 0, la_splits = 0, la_nact = 0;
+    uint64_t                la_origin   = 0;        /* batch frame of the first block of the schedule (priming group) */
+    uint64_t                la_next_t   = 0;        /* batch frame the next launch must carry to continue it */
+    uint32_t                la_prod_cnt[LA_BUFS] = { 0 }, la_cons_cnt[LA_BUFS] = { 0 };    /* the device counters once
+                                                       everything enqueued has run (same for every active instance) */
     std::vector<uint32_t>   h_ring_head;
 
     /* eager pending MAC for synchronous host callers: right after block t has been delivered the
@@ -911,6 +925,11 @@ static int upload_tables(Batch *b, cudaStream_t st)
     for (uint32_t &v : b->h_slot_done)
         v                   = b->frame_seq;
     CU(cudaMemcpyAsync(b->d_slot_done, b->h_slot_done.data(), b->h_slot_done.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    /* ... and no lookahead tail is pending: the schedule restarts with a priming group */
+    CU(cudaMemsetAsync(b->d_la_cnt, 0, 2 * LA_BUFS * b->n * sizeof(uint32_t), st));
+    for (int i = 0; i < LA_BUFS; ++i)
+        b->la_prod_cnt[i] = b->la_cons_cnt[i] = 0;
+    b->la_live          = false;
     /* pageable sources: cudaMemcpyAsync stages them before returning */
     CU(cudaMemcpyAsync(b->d_desc, b->h_desc.data(), b->n * sizeof(InstDesc), cudaMemcpyHostToDevice, st));
     if (!b->active.empty())
@@ -939,6 +958,53 @@ static int ensure_ypart(Batch *b, size_t bytes, cudaStream_t st)
     b->ypart_slot_bytes = want;
     b->pend_ready   = false;
     return B200CONV_OK;
+}
+
+/* the lookahead tail buffer: grown when a schedule (re)starts, never inside one */
+static int ensure_la(Batch *b, size_t bytes, cudaStream_t st)
+{
+    if (bytes <= b->la_T_bytes)
+        return B200CONV_OK;
+    CU(quiesce(b));
+    CU(cudaStreamSynchronize(st));
+    if (b->la_T)
+        cudaFree(b->la_T);
+    b->la_T         = nullptr;
+    b->la_T_bytes   = 0;
+    b->la_live      = false;
+    CU(cudaMalloc(&b->la_T, bytes));
+    b->la_T_bytes   = bytes;
+    return B200CONV_OK;
+}
+
+/* Group size of the k_frame lookahead for a stream of one-frame calls, from what the batch holds:
+ * only launches that stream enough bytes to be bandwidth-bound, bin slices of at least 128 bins
+ * (1 KiB bulk copies), and tails of at least 6K partitions (the head of 2K rows is read every block). */
+static uint32_t lookahead_k(const Batch *b, uint64_t per_frame_bytes)
+{
+    const uint32_t M = 1u << (b->rank - 1);
+    if (b->opt_lookahead >= 0)
+        return uint32_t(b->opt_lookahead);
+    if (per_frame_bytes < LA_MIN_BYTES)
+        return 0;
+    for (uint32_t k = 8; k >= 2; k >>= 1)
+        if ((M / k >= 128) && (b->max_nq >= 8 * size_t(k)))
+            return k;
+    return 0;
+}
+
+/* What a lookahead launch streams per instance: head rows, the bin slices of the tails and the
+ * ring slices of the sliding window, the split rows of T written and read, and the 24 F bytes of
+ * the transform / output of the algorithmic figure (algo_bytes). */
+static uint64_t la_stream_bytes(const Instance &in, uint32_t K, bool use, uint32_t splits)
+{
+    const uint64_t F  = in.F;
+    const size_t q_hi = in.q_lo + in.nq;
+    const size_t qs   = std::max(in.q_lo, std::min(q_hi, size_t(2) * K));
+    const uint64_t nh = use ? (qs - in.q_lo) : in.nq;
+    const uint64_t nt = q_hi - qs;
+    const uint64_t tail = (nt > 0) ? (8 * F / K) * (2 * nt + K - 1) : 0;
+    return 16 * F * nh + tail + 8 * F * splits * (use ? 2 : 1) + 8 * F;
 }
 
 static float2 *ypart_slot(const Batch *b, uint32_t seq)
@@ -1086,6 +1152,8 @@ static int create_impl(b200conv_batch_t **out, int device, size_t instances)
         CU_BRK(cudaMemset(b->d_tickets, 0, FRAME_SLOTS * instances * sizeof(uint32_t)));
         CU_BRK(cudaMalloc(&b->d_slot_done, FRAME_SLOTS * instances * sizeof(uint32_t)));
         CU_BRK(cudaMemset(b->d_slot_done, 0, FRAME_SLOTS * instances * sizeof(uint32_t)));
+        CU_BRK(cudaMalloc(&b->d_la_cnt, 2 * LA_BUFS * instances * sizeof(uint32_t)));
+        CU_BRK(cudaMemset(b->d_la_cnt, 0, 2 * LA_BUFS * instances * sizeof(uint32_t)));
         CU_BRK(cudaHostAlloc(&b->h_error, 64, cudaHostAllocMapped | cudaHostAllocPortable));
         *b->h_error = 0;
         CU_BRK(cudaMalloc(&b->d_ring_head, (instances + 1) * sizeof(uint32_t)));       /* + the chain head (k_mac) */
@@ -1127,6 +1195,8 @@ extern "C" void b200conv_free(b200conv_batch_t *b)
     if (b->d_active)    cudaFree(b->d_active);
     if (b->d_tickets)   cudaFree(b->d_tickets);
     if (b->d_slot_done) cudaFree(b->d_slot_done);
+    if (b->d_la_cnt)    cudaFree(b->d_la_cnt);
+    if (b->la_T)        cudaFree(b->la_T);
     if (b->d_ring_head) cudaFree(b->d_ring_head);
     if (b->h_error)     cudaFreeHost(b->h_error);
     if (b->d_jobs)      cudaFree(b->d_jobs);
@@ -1630,9 +1700,11 @@ static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float 
             hist_unknown(st, b->device);
             b->chain_valid  = false;
             b->ahead_valid  = false;
+            b->la_live      = false;
             b->stats.launches       += 3;
             b->stats.mac_launches   += 1;
             b->stats.mac_algo_bytes += per_frame_bytes * tf;
+            b->stats.mac_stream_bytes += per_frame_bytes * tf;
             b->stats.frames         += uint64_t(nact) * tf;
             used_multi      = true;
             b->pend_ready   = false;
@@ -1641,13 +1713,58 @@ static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float 
         }
         if (fused && (!used_multi))
         {
+            /* Lookahead (kernels.cuh, LA_BUFS): a stream of one-frame calls in uniform mode.  Chosen from
+             * the call pattern and the batch's shape only -- never from pdl, profiling, the stream or the
+             * early-read options -- so that every way of running a stream sums in the same order.  A
+             * synchronous call, a multi-frame call, the general path or any table change ends the schedule;
+             * the next one starts with a priming group (full sums, tails for the group after it). */
+            uint32_t K      = 0;
+            if ((frames == 1) && (!b->eager_call) && (b->reduce.mode == 0))
+                K               = lookahead_k(b, per_frame_bytes);
+            uint64_t launch_bytes = per_frame_bytes;
+            a.la_K          = 0;
+            if (K != 0)
+            {
+                const uint64_t t    = a.t_base + f;
+                if ((!b->la_live) || (b->la_K != K) || (b->la_splits != plan.splits) || (b->la_nact != nact) ||
+                    tables_changed || (b->la_next_t != t))
+                {
+                    TRY(ensure_la(b, size_t(LA_BUFS) * nact * K * plan.splits * F * sizeof(float2), st));
+                    b->la_origin    = t;
+                }
+                const uint64_t rel  = t - b->la_origin;
+                const uint32_t g    = uint32_t((rel / K) % LA_BUFS);
+                a.la_T          = b->la_T;
+                a.la_prod       = b->d_la_cnt;
+                a.la_cons       = b->d_la_cnt + LA_BUFS * b->n;
+                a.la_K          = K;
+                a.la_c          = uint32_t(rel % K);
+                a.la_use        = (rel >= K) ? 1u : 0u;
+                a.la_get        = g;
+                a.la_put        = (g + 1) % LA_BUFS;
+                a.la_put_need   = b->la_cons_cnt[a.la_put];
+                a.la_get_need   = b->la_prod_cnt[a.la_get];
+                if (a.la_use)
+                    b->la_cons_cnt[a.la_get] += 1;
+                b->la_prod_cnt[a.la_put] += plan.splits * plan.tiles;
+                b->la_live      = true;
+                b->la_K         = K;
+                b->la_splits    = plan.splits;
+                b->la_nact      = nact;
+                b->la_next_t    = t + 1;
+                launch_bytes    = 0;
+                for (uint32_t i : b->active)
+                    launch_bytes   += la_stream_bytes(b->inst[i], K, a.la_use != 0, plan.splits);
+            }
+            else
+                b->la_live      = false;
             /* one launch per block for all instances x partitions.  May its input transform run
              * ahead of the launches still in flight on this stream? (FrameHistory) */
             bool early = false, serial = false, dst_clash = false;
             {
                 /* worth it only while the transform is a visible share of the block: a launch that
                  * streams for tens of microseconds hides the chain anyway */
-                const bool capable = (b->opt_pdl != 0) && (!b->profiling) && (per_frame_bytes <= EARLY_MAX_BYTES) &&
+                const bool capable = (b->opt_pdl != 0) && (!b->profiling) && (launch_bytes <= EARLY_MAX_BYTES) &&
                                      ((b->opt_early_src == 2) || ((b->opt_early_src == 1) && (st == b->stream)));
                 const BlockRows in  = { reinterpret_cast<uintptr_t>(src + f * F), stride * sizeof(float), F * sizeof(float), b->n };
                 const BlockRows out = { reinterpret_cast<uintptr_t>(dst + f * F), dst_stride * sizeof(float), F * sizeof(float), b->n };
@@ -1692,12 +1809,15 @@ static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float 
             b->pend_ready   = false;
             b->last_was_frame = (st == b->stream) && (!b->profiling);
             b->stats.launches       += 1;
+            b->stats.mac_stream_bytes += launch_bytes;
         }
         else
         {
             MacPlan sp      = plan;
             sp.sh.bias      = 0;
             b->pend_ready   = false;
+            b->la_live      = false;
+            b->stats.mac_stream_bytes += per_frame_bytes;
             const bool ahead = (b->rank >= 14) && (b->opt_pdl != 0) && (!b->profiling) && (b->opt_chain_ahead != 0) && (frames == 1);
             if (ahead)
             {
@@ -1896,6 +2016,7 @@ static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const 
     const size_t F      = size_t(1) << (b->rank - 1);
     TRY(upload_tables(b, st));
     hist_reset(st, b->device);          /* every CTA of the job-list form waits for all earlier launches */
+    b->la_live          = false;        /* a lookahead schedule restarts with a priming group */
     std::vector<size_t> &pos = b->g_pos;
     std::vector<Job> &jobs = b->g_jobs;
     for (uint32_t i : b->active)
@@ -2043,6 +2164,7 @@ static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const 
         {
             b->stats.mac_launches   += 1;
             b->stats.mac_algo_bytes += bytes;
+            b->stats.mac_stream_bytes += bytes;
         }
     }
 
@@ -2257,6 +2379,7 @@ static int process_general_staged(Batch *b, float *dst, size_t dst_stride, const
             b->stats.launches       += 2;
             b->stats.mac_launches   += 1;
             b->stats.mac_algo_bytes += bytes;
+            b->stats.mac_stream_bytes += bytes;
         }
     }
 
@@ -2691,6 +2814,8 @@ extern "C" int b200conv_set_option(b200conv_batch_t *b, const char *name, int va
     else if (!strcmp(name, "eager") && (value >= 0) && (value <= 1))        b->opt_eager = value;
     else if (!strcmp(name, "early_pend") && (value >= 0) && (value <= 2))   b->opt_early_pend = value;
     else if (!strcmp(name, "early_src") && (value >= 0) && (value <= 2))    b->opt_early_src = value;
+    else if (!strcmp(name, "lookahead") && ((value == -1) || (value == 0) || (value == 2) || (value == 4) || (value == 8)))
+        b->opt_lookahead = value;
     else if (!strcmp(name, "multi_frame") && ((value == 0) || (value == 1) || (value == 2) || (value == 4) || (value == 8)))
         b->opt_multi = (value == 1) ? 0 : value;
     else

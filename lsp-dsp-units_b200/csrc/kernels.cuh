@@ -116,6 +116,16 @@ struct StepArgs                     /* by-value kernel argument */
     uint32_t        rank;
     uint32_t        frame0;         /* uniform mode: first frame (within the call) of this launch   */
     uint32_t        flags;
+    /* k_frame lookahead (one-frame-per-call streams, see LA_BUFS): la_K = 0 -> off */
+    float2         *la_T;           /* [LA_BUFS][n_jobs][la_K][splits][M] tail sums T of a group's blocks    */
+    uint32_t       *la_prod;        /* [LA_BUFS][n_cap] CTAs that have written their tail rows into that buffer */
+    uint32_t       *la_cons;        /* [LA_BUFS][n_cap] launch tails that have read their T rows from it     */
+    uint32_t        la_K;           /* group size K (2, 4, 8)                                               */
+    uint32_t        la_c;           /* this launch's block within its group: it streams bin slice la_c      */
+    uint32_t        la_use;         /* T of this block is complete: the launch sums partitions q < 2K only  */
+    uint32_t        la_put, la_get; /* buffer this launch writes (next group) / reads (its own group)       */
+    uint32_t        la_put_need;    /* la_cons[la_put] must reach this before the first tail-row write      */
+    uint32_t        la_get_need;    /* la_prod[la_get] must reach this before the T rows are read           */
 };
 
 enum { INV_FULL = 1, STEP_FROM_Q1 = 2, STEP_HEAD_ONLY = 4,
@@ -172,6 +182,23 @@ enum { INV_FULL = 1, STEP_FROM_Q1 = 2, STEP_HEAD_ONLY = 4,
  *   completion     the tail CTAs execute griddepcontrol.wait as their LAST instruction, so launch
  *                  s completes after launch s - 1 (stream order for whatever follows). */
 constexpr int FRAME_SLOTS      = 4;
+/* Lookahead for streams of one-frame calls (k_frame, la_K = K > 0).  Blocks are grouped K at a time
+ * (group g = blocks t0 .. t0 + K - 1).  y_t needs  head_t = sum_{q < 2K} G_q X_{t-q}  and the tail
+ * T_t = sum_{q >= 2K} G_q X_{t-q}, which reads frames <= t - 2K only.  For every block of group g + 1
+ * that is a frame <= t0 - 1, so the K launches of group g compute the tails of group g + 1, launch
+ * t0 + c the bin slice [c M / K, (c + 1) M / K) of all K of them: each IR spectrum row is streamed
+ * once per group instead of once per block.  A launch sums its own head (or, when the tails of its
+ * group are not complete -- the first group after any interruption -- every partition), adds the
+ * split rows of its T (written by the K launches before it), and inverts.  Every T value has one
+ * writer and the summation order is fixed: results do not depend on timing or on the overlap.
+ * Ordering (all waits bounded, per instance, sequence counts the host predicts):
+ *   T complete   la_prod[buf] counts producer CTAs (st.release after the rows); the tail CTA of a
+ *                consumer polls it before reading its T rows (launch t0 + K reads rows that launch
+ *                t0 + K - 1 may still be writing);
+ *   T reuse      LA_BUFS = 3 buffers rotate by group; la_cons[buf] counts the consumers that have
+ *                read their rows; a producer polls it before its first row write (the last reader
+ *                of a buffer is K + 1 launches before its next writer, so it is long done there). */
+constexpr int LA_BUFS          = 3;
 constexpr int REDUCE_MAX_WORLD = 8;
 constexpr int REDUCE_DEPTH     = 4;
 struct ReduceArgs
@@ -1005,8 +1032,10 @@ enum { INV_OLA = 1, INV_PRESUMMED = 2, INV_STAGED = 4 };
 template <int RANK, bool PP, int RG = 8, int TT = 0, int MODE = 0, bool WM = (RANK >= 12), int NHO = 0, bool TWC = false>     /* RG: partial rows loaded per round (registers) */
 __device__ __forceinline__ void inv_body(float2 *A, float2 *B, const float2 *yp, uint32_t splits,
                                          float *dst, const float2 *twg, const float2 *tw, bool full, int tid,
-                                         int only_pass = -1, const float2 *g0 = nullptr, const float2 *x0 = nullptr)
+                                         int only_pass = -1, const float2 *g0 = nullptr, const float2 *x0 = nullptr,
+                                         const float2 *yp2 = nullptr, uint32_t splits2 = 0)
 {
+    /* yp2, splits2: more rows to add after the `splits` rows of yp (k_frame lookahead: the block's T rows) */
     /* g0, x0 (rows summed from global memory only, !PP): one more term, g0[k] * x0[k] -- partition 0
      * against the block's own spectrum (STEP_Q0_IN_INV); bin 0 packs two real values (DC, Nyquist) */
     const float2 *twx       = TWC ? twg : tw;      /* TWC: `tw` is the compact pass table (fft_smem) */
@@ -1038,26 +1067,32 @@ __device__ __forceinline__ void inv_body(float2 *A, float2 *B, const float2 *yp,
             {
                 const int ca = c0 + tid, cb = c0 + T + tid;
                 float4 sa = make_float4(0.0f, 0.0f, 0.0f, 0.0f), sb = sa;
-                for (uint32_t s0 = 0; s0 < splits; s0 += RG)
+                #pragma unroll 1
+                for (int set = 0; set < 2; ++set)
+                {
+                const float2 *yr    = set ? yp2 : yp;
+                const uint32_t nr   = set ? splits2 : splits;
+                for (uint32_t s0 = 0; s0 < nr; s0 += RG)
                 {
                     float4 va[RG], vb[RG];
                     #pragma unroll
                     for (int r = 0; r < RG; ++r)
                     {
-                        uint32_t row = min(s0 + r, splits - 1);     /* clamp: the extra loads are dropped below */
-                        const float4 *rp = reinterpret_cast<const float4 *>(yp + uint64_t(row) * M);
+                        uint32_t row = min(s0 + r, nr - 1);         /* clamp: the extra loads are dropped below */
+                        const float4 *rp = reinterpret_cast<const float4 *>(yr + uint64_t(row) * M);
                         va[r]       = ld_cg_f4(rp + ca);
                         vb[r]       = ld_cg_f4(rp + cb);
                     }
                     #pragma unroll
                     for (int r = 0; r < RG; ++r)
                     {
-                        if (s0 + r < splits)
+                        if (s0 + r < nr)
                         {
                             sa.x += va[r].x; sa.y += va[r].y; sa.z += va[r].z; sa.w += va[r].w;
                             sb.x += vb[r].x; sb.y += vb[r].y; sb.z += vb[r].z; sb.w += vb[r].w;
                         }
                     }
+                }
                 }
                 ysum[ca]    = sa;
                 ysum[cb]    = sb;
@@ -1102,9 +1137,9 @@ __device__ __forceinline__ void inv_body(float2 *A, float2 *B, const float2 *yp,
                 #pragma unroll
                 for (int u = 0; u < UB; ++u)
                     yk[u] = ym[u] = make_float2(0.0f, 0.0f);
-                for (uint32_t s = 0; s < splits; ++s)
+                for (uint32_t s = 0; s < splits + splits2; ++s)
                 {
-                    const float2 *row = yp + uint64_t(s) * M;
+                    const float2 *row = (s < splits) ? yp + uint64_t(s) * M : yp2 + uint64_t(s - splits) * M;
                     #pragma unroll
                     for (int u = 0; u < UB; ++u)
                     {
@@ -1468,6 +1503,14 @@ __device__ __forceinline__ uint64_t stream_policy()
 {
     uint64_t policy;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+    return policy;
+}
+
+/* rows that later launches read again (k_frame lookahead: the head rows q < 2K) */
+__device__ __forceinline__ uint64_t keep_policy()
+{
+    uint64_t policy;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(policy));
     return policy;
 }
 
@@ -2303,6 +2346,13 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
 
     uint32_t qa             = max(job.qa, d.q_lo);
     uint32_t qb             = min(job.qb, d.q_lo + d.nq);
+    /* lookahead (LA_BUFS): this launch streams bin slice la_c of the tails [qs, qb) of the next
+     * group's blocks; its own head is [qa, qs) when its T is complete, else every partition */
+    const uint32_t LK       = GEN ? 0u : a.la_K;
+    const uint32_t qs       = (LK != 0) ? max(qa, min(qb, 2u * LK)) : qb;
+    const uint32_t qe       = qb;
+    if ((LK != 0) && a.la_use)
+        qb                      = qs;
     uint32_t nq             = ((qb > qa) && ((!GEN) || (job.flags & JOB_MAC))) ? (qb - qa) : 0;
     uint32_t c0, c1;
     chunk_range(nq, split, a.splits, sh.bias, c0, c1);
@@ -2320,6 +2370,31 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
     const float2 *Xt        = d.ring + uint64_t(tile) * TB;
     const uint32_t row_bytes = TB * uint32_t(sizeof(float2));
     const uint64_t l2_stream = stream_policy();
+    /* the head rows of a lookahead launch are read again by the next 2K - 1 launches: keep them in L2 */
+    const uint64_t l2_head  = (LK != 0) ? keep_policy() : l2_stream;
+
+    /* Lookahead tail, as a "virtual row" of M bins: segment j (W = M / K bins) of the row of partition q
+     * is  G_q[slice] * X_{t0 + K + j - q}[slice]  -- the same multiply-add loop as the head rows.  A
+     * tile of TB virtual bins covers nj segments j0 .. j0 + nj - 1 (or a part of one: Wg bins at offset
+     * p0 of the slice).  One stage holds QT partitions: QT G slices, then the QT + nj - 1 ring slices
+     * of frames fmax, fmax - 1, ... (ascending ring slots), fmax = t0 + K + j0 + nj - 1 - q. */
+    uint32_t tq0 = 0, tq1 = 0, n_titer = 0, QT = 1, Wg = 0, Wc4 = 1, nj = 1, j0 = 0, p0 = 0;
+    if (LK != 0)
+    {
+        const uint32_t W    = M / LK;
+        Wg                  = min(W, TB);
+        Wc4                 = Wg / 2;
+        nj                  = max(1u, TB / W);
+        j0                  = (tile * TB) / W;
+        p0                  = (tile * TB) % W;
+        QT                  = max(1u, ((2u * stage_elems) / Wg - (nj - 1)) / 2);
+        uint32_t e0, e1;
+        chunk_range(qe - qs, split, a.splits, sh.bias, e0, e1);
+        tq0                 = qs + e0;
+        tq1                 = qs + e1;
+        n_titer             = (tq1 - tq0 + QT - 1) / QT;
+    }
+    const uint32_t t0       = job.tlo - a.la_c;                    /* first block of this launch's group */
 
     /* Stage-ring bookkeeping is incremental (next stage buffer, next ring slot): no integer
      * division inside the streaming loop.  `issued` = stages fetched so far. */
@@ -2327,8 +2402,40 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
     uint32_t issued = 0, f_s = 0;
     uint32_t f_slot         = slot_q0 + late * QB;
     if (f_slot >= d.S)      f_slot -= d.S;
+    uint32_t t_issued = 0;
     auto issue_next = [&]()                     /* thread 0 only */
     {
+        if (t_issued < n_titer)
+        {
+            /* a lookahead tail stage: partitions q .. q + rows - 1 of bin slice la_c */
+            const uint32_t q    = tq0 + t_issued * QT;
+            const uint32_t rows = min(QT, tq1 - q);
+            if (t_issued == 0)
+            {
+                /* the tails read frames <= t0 - 1 (the oldest one, t0 + K - (bins + 1) + 1, is newer than
+                 * the oldest frame a launch without lookahead reads: the ring size is unchanged) */
+                wait_ge<false>(a.ring_head + job.inst, t0, a.error, SPIN_ERR_RING);
+                asm volatile("fence.proxy.async;" ::: "memory");
+            }
+            const uint32_t nx   = rows + nj - 1;
+            const uint32_t sb   = Wg * uint32_t(sizeof(float2));
+            float2 *g           = stages + size_t(f_s) * 2 * stage_elems;
+            float2 *x           = g + size_t(QT) * Wg;
+            const uint64_t boff = uint64_t(a.la_c) * (M / LK) + p0;
+            mbar_expect_tx(&full[f_s], (rows + nx) * sb);
+            for (uint32_t r = 0; r < rows; ++r)
+                bulk_g2s(g + size_t(r) * Wg, d.G + uint64_t(q + r - d.q_lo) * M + boff, sb, &full[f_s], l2_stream);
+            /* frame fmax = t0 + K + j0 + nj - 1 - q lives in slot (slot0 + t - fmax) mod S, t - fmax >= 1 */
+            uint32_t sl         = uint32_t((uint64_t(job.slot0) + (a.la_c + q + 1u - (LK + j0 + nj))) % d.S);
+            for (uint32_t i = 0; i < nx; ++i)
+            {
+                bulk_g2s(x + size_t(i) * Wg, d.ring + uint64_t(sl) * M + boff, sb, &full[f_s], l2_stream);
+                if (++sl == d.S)    sl = 0;
+            }
+            ++t_issued;
+            if (++f_s == NS)    f_s = 0;
+            return;
+        }
         uint32_t stg;
         if (issued < n_iter - late)
         {
@@ -2357,11 +2464,11 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         float2 *g       = stages + size_t(f_s) * 2 * stage_elems;
         float2 *x       = g + stage_elems;
         mbar_expect_tx(&full[f_s], 2u * rows * row_bytes);
-        bulk_g2s(g, Gt + uint64_t(q - d.q_lo) * M, rows * row_bytes, &full[f_s], l2_stream);
+        bulk_g2s(g, Gt + uint64_t(q - d.q_lo) * M, rows * row_bytes, &full[f_s], l2_head);
         uint32_t n1     = min(rows, d.S - f_slot);
-        bulk_g2s(x, Xt + uint64_t(f_slot) * M, n1 * row_bytes, &full[f_s], l2_stream);
+        bulk_g2s(x, Xt + uint64_t(f_slot) * M, n1 * row_bytes, &full[f_s], l2_head);
         if (n1 < rows)
-            bulk_g2s(x + size_t(n1) * TB, Xt, (rows - n1) * row_bytes, &full[f_s], l2_stream);
+            bulk_g2s(x + size_t(n1) * TB, Xt, (rows - n1) * row_bytes, &full[f_s], l2_head);
         ++issued;
         if (++f_s == NS)    f_s = 0;
         f_slot         += QB;
@@ -2369,7 +2476,7 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
     };
 
     if (tid == 0)
-        while ((issued < NS) && (issued < n_main))
+        while ((t_issued + issued < NS) && (t_issued + issued < n_titer + n_main))
             issue_next();
 
     float *po               = nullptr;
@@ -2475,6 +2582,79 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         ++c_n;
         if (++c_s == NS)        { c_s = 0; c_par ^= 1u; }
     };
+
+    if (LK != 0)
+    {
+        /* the lookahead tail: virtual columns lc = tid + v T of this tile, see above */
+        uint32_t gofs[MAC_VPT], xofs[MAC_VPT];
+        float tdn[MAC_VPT];
+        #pragma unroll
+        for (int v = 0; v < MAC_VPT; ++v)
+        {
+            const uint32_t lc   = tid + v * T;
+            gofs[v]             = lc % Wc4;
+            xofs[v]             = (nj - 1 - lc / Wc4) * Wc4 + gofs[v];
+            tdn[v]              = 0.0f;
+        }
+        uint32_t t_cons = 0;
+        for (uint32_t it = 0; it < n_titer; ++it)
+        {
+            const uint32_t rows = min(QT, tq1 - (tq0 + t_cons * QT));
+            mbar_wait(&full[c_s], c_par);
+            const float4 *g4 = reinterpret_cast<const float4 *>(stages + size_t(c_s) * 2 * stage_elems);
+            const float4 *x4 = g4 + QT * Wc4;
+            for (uint32_t r = 0; r < rows; ++r)
+            {
+                #pragma unroll
+                for (int v = 0; v < MAC_VPT; ++v)
+                {
+                    float4 g    = g4[r * Wc4 + gofs[v]];
+                    float4 x    = x4[r * Wc4 + xofs[v]];
+                    acc[v].x    = fmaf(g.x, x.x, acc[v].x);
+                    acc[v].y    = fmaf(g.x, x.y, acc[v].y);
+                    acc[v].z    = fmaf(g.z, x.z, acc[v].z);
+                    acc[v].w    = fmaf(g.z, x.w, acc[v].w);
+                    acc[v].x    = fmaf(-g.y, x.y, acc[v].x);
+                    acc[v].y    = fmaf(g.y, x.x, acc[v].y);
+                    acc[v].z    = fmaf(-g.w, x.w, acc[v].z);
+                    acc[v].w    = fmaf(g.w, x.z, acc[v].w);
+                    tdn[v]      = fmaf(g.y, x.y, tdn[v]);
+                }
+            }
+            ++t_cons;
+            if (++c_s == NS)        { c_s = 0; c_par ^= 1u; }
+            __syncthreads();
+            if ((tid == 0) && ((t_issued < n_titer) || (issued < n_main)))
+                issue_next();
+        }
+        /* bin 0 (DC, Nyquist) of the spectrum opens slice 0 of every segment */
+        #pragma unroll
+        for (int v = 0; v < MAC_VPT; ++v)
+            if ((a.la_c == 0) && (p0 == 0) && (gofs[v] == 0))
+            {
+                acc[v].x       += tdn[v];
+                acc[v].y        = tdn[v];
+            }
+        /* buffer la_put was last read by the blocks of the group LA_BUFS - 1 before the next one */
+        if (tid == 0)
+            wait_ge<false>(a.la_cons + size_t(a.la_put) * a.n_cap + job.inst, a.la_put_need, a.error, SPIN_ERR_RING);
+        __syncthreads();
+        float2 *tb      = a.la_T + uint64_t(a.la_put) * a.n_jobs * LK * a.splits * M
+                                 + uint64_t(a.la_c) * (M / LK) + p0;
+        #pragma unroll
+        for (int v = 0; v < MAC_VPT; ++v)
+        {
+            const uint32_t j    = j0 + (tid + v * T) / Wc4;
+            float4 *tp          = reinterpret_cast<float4 *>(tb + ((uint64_t(jobi) * LK + j) * a.splits + split) * M) + gofs[v];
+            __stcg(tp, acc[v]);
+            acc[v]              = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        }
+        __threadfence();
+        __syncthreads();
+        if (tid == 0)
+            asm volatile("red.release.gpu.global.add.u32 [%0], 1;"
+                         :: "l"(a.la_prod + size_t(a.la_put) * a.n_cap + job.inst) : "memory");
+    }
 
     for (uint32_t it = 0; it < n_main; ++it)
     {
@@ -2651,7 +2831,28 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
                 cp_async4(po + 2 * AW + i, job.psrc2 + i);
             }
         }
-        inv_body<RANK, TAIL_PP, TAIL_RG, int(T)>(wa, wb, ysum, nsum, job.dst, a.tw, tw, false, int(tid));
+        /* lookahead: the block's tail T, split rows written by the K launches before this one */
+        const float2 *yT    = nullptr;
+        uint32_t nT         = 0;
+        if ((LK != 0) && a.la_use)
+        {
+            if (tid == 0)
+                wait_ge<false>(a.la_prod + size_t(a.la_get) * a.n_cap + job.inst, a.la_get_need, a.error, SPIN_ERR_RING);
+            __syncthreads();
+            yT                  = a.la_T + ((uint64_t(a.la_get) * a.n_jobs + jobi) * LK + a.la_c) * a.splits * M;
+            nT                  = a.splits;
+        }
+        inv_body<RANK, TAIL_PP, TAIL_RG, int(T)>(wa, wb, ysum, nsum, job.dst, a.tw, tw, false, int(tid),
+                                                 -1, nullptr, nullptr, yT, nT);
+        if (nT != 0)
+        {
+            /* the T rows have been read: the buffer may take the next group's tails */
+            __threadfence();
+            __syncthreads();
+            if (tid == 0)
+                asm volatile("red.release.gpu.global.add.u32 [%0], 1;"
+                             :: "l"(a.la_cons + size_t(a.la_get) * a.n_cap + job.inst) : "memory");
+        }
         if (GEN)
             FRAME_STAMP(7);
         if (GEN && spread)
