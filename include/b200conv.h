@@ -488,6 +488,26 @@ size_t  b200conv_ss_handlers(const b200conv_ss_t *s);
  *                               input history is discarded.  On B200CONV_ERR_ARG / _ERR_NOMEM nothing
  *                               changes (the old routes and history stay).  Ordered after every call
  *                               already enqueued on the object; synchronous
+ *   b200conv_mx_set_irs         replaces the IRs of some routes and KEEPS the input history: route
+ *                               route[k] (its index in the last set_routes) gets ir[k][0 .. length[k])
+ *                               (HOST pointers, copied to page-locked staging before the call returns).
+ *                               With k counting samples from the first sample of the next process call
+ *                               and w(k) = min(1, (k + 1) / fade) (w = 1 when fade == 0: a hard switch),
+ *                               a changed route contributes (1 - w) h_old (*) x + w h_new (*) x, both
+ *                               over the whole history since set_routes / clear; once the fade is over
+ *                               the new IRs stay.  B200CONV_ERR_ARG: route out of range or twice, NULL
+ *                               or empty IR, or an IR of more partitions than the ring reaches
+ *                               (ceil(length / F) + 1 > the longest route's at set_routes: use
+ *                               set_routes); B200CONV_ERR_STATE: a fade is in progress.  On any error
+ *                               nothing changes; count == 0 is a no-op; a one-tap zero IR fades a route
+ *                               out.  Enqueued on `stream` (NULL = the object's own) like
+ *                               process_device, with stream-ordered allocations; the host waits only
+ *                               while the previous call's staging is still being uploaded.  During a
+ *                               fade each launch group runs the delta routes (G_new - G_old) into
+ *                               extra outputs and one blend launch.  clear ends a fade with the new
+ *                               IRs in place; set_routes discards it
+ *   b200conv_mx_fade_remaining  samples of the fade not yet covered by the calls enqueued so far
+ *                               (0: no fade); host arithmetic, never waits
  *   b200conv_mx_clear           discards the input history, keeps the routes
  *   b200conv_mx_process_device  src: DEVICE matrix [inputs][src_stride], dst: DEVICE matrix
  *                               [outputs][dst_stride] floats; count must be a multiple of F (0 = no-op;
@@ -506,6 +526,9 @@ int     b200conv_mx_create(b200conv_mx_t **out, int device, size_t inputs, size_
 void    b200conv_mx_free(b200conv_mx_t *m);
 int     b200conv_mx_set_routes(b200conv_mx_t *m, size_t count, const size_t *input, const size_t *output,
                                const float *const *ir, const size_t *length);
+int     b200conv_mx_set_irs(b200conv_mx_t *m, size_t count, const size_t *route,
+                            const float *const *ir, const size_t *length, size_t fade, void *stream);
+size_t  b200conv_mx_fade_remaining(const b200conv_mx_t *m);
 int     b200conv_mx_clear(b200conv_mx_t *m);
 int     b200conv_mx_process_device(b200conv_mx_t *m, float *dst, size_t dst_stride, const float *src,
                                    size_t src_stride, size_t count, void *stream);

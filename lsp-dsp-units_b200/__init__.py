@@ -165,6 +165,9 @@ _SIGNATURES = {
     "b200conv_mx_free": (None, [_VP]),
     "b200conv_mx_set_routes": (ctypes.c_int, [_VP, _SZ, ctypes.POINTER(_SZ), ctypes.POINTER(_SZ), ctypes.POINTER(_FP),
                                               ctypes.POINTER(_SZ)]),
+    "b200conv_mx_set_irs": (ctypes.c_int, [_VP, _SZ, ctypes.POINTER(_SZ), ctypes.POINTER(_FP), ctypes.POINTER(_SZ),
+                                           _SZ, _VP]),
+    "b200conv_mx_fade_remaining": (_SZ, [_VP]),
     "b200conv_mx_clear": (ctypes.c_int, [_VP]),
     "b200conv_mx_process_device": (ctypes.c_int, [_VP, _VP, _SZ, _VP, _SZ, _SZ, _VP]),
     "b200conv_mx_process_planar": (ctypes.c_int, [_VP, _VP, _SZ, _VP, _SZ, _SZ]),
@@ -730,6 +733,22 @@ class MatrixConvolver:
         _check(lib().b200conv_mx_set_routes(self._h, n, (_SZ * n)(*[int(r[0]) for r in routes]),
                                             (_SZ * n)(*[int(r[1]) for r in routes]),
                                             (_FP * n)(*[_ptr(h) for h in irs]), (_SZ * n)(*[h.size for h in irs])))
+
+    def set_irs(self, changes, fade=0, stream=None):
+        """``changes``: ``[(route, ir), ...]`` with ``route`` the index in the last ``set_routes``.  Keeps the
+        input history and crossfades each changed route from its old IR to the new one over ``fade``
+        samples, starting with the next call (0: a hard switch).  Stream-ordered like ``process_device``
+        (``stream`` None = the object's own stream); does not wait for the device."""
+        changes = list(changes)
+        n = len(changes)
+        irs = [np.ascontiguousarray(h, dtype=np.float32).ravel() for _, h in changes]
+        _check(lib().b200conv_mx_set_irs(self._h, n, (_SZ * n)(*[int(c[0]) for c in changes]),
+                                         (_FP * n)(*[_ptr(h) for h in irs]), (_SZ * n)(*[h.size for h in irs]),
+                                         int(fade), stream))
+
+    def fade_remaining(self):
+        """Samples of the crossfade not yet covered by the calls enqueued so far (0: none running)."""
+        return int(lib().b200conv_mx_fade_remaining(self._h))
 
     def clear(self):
         _check(lib().b200conv_mx_clear(self._h))

@@ -250,6 +250,70 @@ k_mx_mac(const MxArgs a)
         asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
+/* ---- impulse-response replacement with a crossfade (b200conv_mx_set_irs) --------------------------
+ * The ring holds input spectra only and no state crosses a block boundary, so by linearity
+ *     y_o = IFFT(A + B_old) + w(n) * IFFT(B_delta),   B_delta = sum_q (G_new - G_old)_q X_{t-q}
+ * where A sums the unchanged routes into o and B_old the old IRs of the changed ones.  The delta terms
+ * are extra "delta routes" into extra "delta outputs" of k_mx_mac and k_inv; the two kernels below
+ * ingest the new IRs and blend the delta outputs into the real ones. */
+
+struct FoldDeltaDesc                /* one changed route */
+{
+    float2         *G;              /* [bins + 1][M] folded spectra of the new IR                  */
+    float2         *D;              /* [nd][M] G_new - G_old, each zero-extended to nd rows; NULL:
+                                       no fade, G_new only (nd = bins + 1)                           */
+    const float2   *G_old;          /* [nq_old][M] the route's current folded spectra               */
+    uint64_t        h_row;          /* first row of the route in the H slab                         */
+    uint32_t        bins;           /* partitions of the new IR                                     */
+    uint32_t        nq_old;
+    uint32_t        nd;             /* max(bins + 1, nq_old)                                         */
+    uint32_t        pad;
+};
+
+/* k_fold_many's fold of H into G_new, and G_new - G_old, in one pass */
+__global__ void k_fold_delta(const FoldDeltaDesc *desc, uint32_t n, const float2 *H, uint32_t M)
+{
+    for (uint32_t i = blockIdx.z; i < n; i += gridDim.z)
+    {
+        const FoldDeltaDesc d = desc[i];
+        const float2 *Hi    = H + d.h_row * M;
+        for (uint32_t q = blockIdx.y; q < d.nd; q += gridDim.y)
+        for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < M; k += gridDim.x * blockDim.x)
+        {
+            float2 g        = make_float2(0.0f, 0.0f);
+            if (q <= d.bins)
+            {
+                float2 cur      = (q < d.bins) ? Hi[uint64_t(q) * M + k] : make_float2(0.0f, 0.0f);
+                float2 prev     = (q > 0) ? Hi[uint64_t(q - 1) * M + k] : make_float2(0.0f, 0.0f);
+                float sgn       = (k & 1) ? -1.0f : 1.0f;
+                g               = make_float2(cur.x + sgn * prev.x, cur.y + sgn * prev.y);
+                d.G[uint64_t(q) * M + k] = g;
+            }
+            if (d.D == nullptr)
+                continue;
+            const float2 o  = (q < d.nq_old) ? d.G_old[uint64_t(q) * M + k] : make_float2(0.0f, 0.0f);
+            d.D[uint64_t(q) * M + k] = make_float2(g.x - o.x, g.y - o.y);
+        }
+    }
+}
+
+/* dst[omap[d]][z * F + n] += w(k) * delta[z][d][n] with k = k0 + z * F + n the sample index since the
+ * fade began and w(k) = min(1, (k + 1) / fade): exact wherever the fade ends.  grid = (., deltas, frames);
+ * launched after the k_inv that wrote both, so dst == src calls stay safe. */
+__global__ void k_mx_blend(float *dst, uint64_t dst_stride, const float *delta, const uint32_t *omap,
+                           uint32_t deltas, uint32_t F, uint64_t k0, uint64_t fade)
+{
+    const uint32_t di   = blockIdx.y, z = blockIdx.z;
+    const float *dz     = delta + (uint64_t(z) * deltas + di) * F;
+    float *y            = dst + uint64_t(omap[di]) * dst_stride + uint64_t(z) * F;
+    for (uint32_t n = blockIdx.x * blockDim.x + threadIdx.x; n < F; n += gridDim.x * blockDim.x)
+    {
+        const uint64_t k    = k0 + uint64_t(z) * F + n;
+        const float w       = (k + 1 >= fade) ? 1.0f : float(double(k + 1) / double(fade));
+        y[n]                = fmaf(w, dz[n], y[n]);
+    }
+}
+
 }   /* namespace b200conv */
 
 #endif /* B200CONV_MATRIX_CUH_ */
