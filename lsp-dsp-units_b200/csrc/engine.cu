@@ -993,17 +993,29 @@ static uint32_t lookahead_k(const Batch *b, uint64_t per_frame_bytes)
     return 0;
 }
 
-/* What a lookahead launch streams per instance: head rows, the bin slices of the tails and the
- * ring slices of the sliding window, the split rows of T written and read, and the 24 F bytes of
+/* What a lookahead launch copies per instance: head rows; per k_frame CTA (split x bin tile) the G
+ * slices of its tail partitions and its ring window, which holds nj - 1 slices more (nj = segments
+ * of the tile, kernels.cuh frame_body); the split rows of T written and read; and the 24 F bytes of
  * the transform / output of the algorithmic figure (algo_bytes). */
-static uint64_t la_stream_bytes(const Instance &in, uint32_t K, bool use, uint32_t splits)
+static uint64_t la_stream_bytes(const Instance &in, uint32_t K, bool use, const MacShape &sh, uint32_t splits)
 {
     const uint64_t F  = in.F;
     const size_t q_hi = in.q_lo + in.nq;
     const size_t qs   = std::max(in.q_lo, std::min(q_hi, size_t(2) * K));
     const uint64_t nh = use ? (qs - in.q_lo) : in.nq;
-    const uint64_t nt = q_hi - qs;
-    const uint64_t tail = (nt > 0) ? (8 * F / K) * (2 * nt + K - 1) : 0;
+    const uint32_t nt = uint32_t(q_hi - qs);
+    const uint64_t W  = F / K;
+    const uint64_t Wg = std::min<uint64_t>(W, sh.TB);
+    const uint64_t nj = std::max<uint64_t>(1, sh.TB / W);
+    uint64_t slices   = 0;
+    for (uint32_t s = 0; s < splits; ++s)
+    {
+        uint32_t e0, e1;
+        chunk_range(nt, s, splits, sh.bias, e0, e1);
+        if (e1 > e0)
+            slices         += 2 * uint64_t(e1 - e0) + nj - 1;
+    }
+    const uint64_t tail = (F / sh.TB) * slices * 8 * Wg;
     return 16 * F * nh + tail + 8 * F * splits * (use ? 2 : 1) + 8 * F;
 }
 
@@ -1754,7 +1766,7 @@ static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float 
                 b->la_next_t    = t + 1;
                 launch_bytes    = 0;
                 for (uint32_t i : b->active)
-                    launch_bytes   += la_stream_bytes(b->inst[i], K, a.la_use != 0, plan.splits);
+                    launch_bytes   += la_stream_bytes(b->inst[i], K, a.la_use != 0, plan.sh, plan.splits);
             }
             else
                 b->la_live      = false;

@@ -23,6 +23,7 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 
 namespace b200conv
 {
@@ -1677,7 +1678,7 @@ struct MacShape
 };
 
 /* Partition chunk [c0, c1) (relative to the job's first partition) of split `split`. */
-__device__ __forceinline__ void chunk_range(uint32_t nq, uint32_t split, uint32_t splits, uint32_t bias,
+__host__ __device__ __forceinline__ void chunk_range(uint32_t nq, uint32_t split, uint32_t splits, uint32_t bias,
                                             uint32_t &c0, uint32_t &c1)
 {
     uint32_t even   = nq / splits;
@@ -2283,6 +2284,20 @@ __device__ __forceinline__ void partial_outputs(const float *cur, const float *h
 /* so a src that an earlier launch produced (two batches cascaded on one stream, or a batch fed   */
 /* its own dst) is final when it is read, whoever that producer was.                             */
 
+/* acc += g * x for two packed complex bins; dn += Im g * Im x (the bin-0 Nyquist fix-up) */
+__device__ __forceinline__ void cmac(float4 &acc, float &dn, const float4 g, const float4 x)
+{
+    acc.x           = fmaf(g.x, x.x, acc.x);
+    acc.y           = fmaf(g.x, x.y, acc.y);
+    acc.z           = fmaf(g.z, x.z, acc.z);
+    acc.w           = fmaf(g.z, x.w, acc.w);
+    acc.x           = fmaf(-g.y, x.y, acc.x);
+    acc.y           = fmaf(g.y, x.x, acc.y);
+    acc.z           = fmaf(-g.w, x.w, acc.z);
+    acc.w           = fmaf(g.w, x.z, acc.w);
+    dn              = fmaf(g.y, x.y, dn);
+}
+
 template <int RANK>
 struct FrameCfg
 {
@@ -2369,30 +2384,38 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
     const float2 *Gt        = d.G + uint64_t(tile) * TB;            /* row r at Gt + r * M */
     const float2 *Xt        = d.ring + uint64_t(tile) * TB;
     const uint32_t row_bytes = TB * uint32_t(sizeof(float2));
-    const uint64_t l2_stream = stream_policy();
-    /* the head rows of a lookahead launch are read again by the next 2K - 1 launches: keep them in L2 */
-    const uint64_t l2_head  = (LK != 0) ? keep_policy() : l2_stream;
 
     /* Lookahead tail, as a "virtual row" of M bins: segment j (W = M / K bins) of the row of partition q
-     * is  G_q[slice] * X_{t0 + K + j - q}[slice]  -- the same multiply-add loop as the head rows.  A
-     * tile of TB virtual bins covers nj segments j0 .. j0 + nj - 1 (or a part of one: Wg bins at offset
-     * p0 of the slice).  One stage holds QT partitions: QT G slices, then the QT + nj - 1 ring slices
-     * of frames fmax, fmax - 1, ... (ascending ring slots), fmax = t0 + K + j0 + nj - 1 - q. */
-    uint32_t tq0 = 0, tq1 = 0, n_titer = 0, QT = 1, Wg = 0, Wc4 = 1, nj = 1, j0 = 0, p0 = 0;
+     * is  G_q[slice] * X_{t0 + K + j - q}[slice]  -- the same multiply-add as the head rows.  A tile of
+     * TB virtual bins covers nj segments j0 .. j0 + nj - 1 (or a part of one: Wg bins at offset p0 of
+     * the slice).  The CTA's partitions tq0 .. tq1 - 1 go QT per stage.  Its ring slices form ONE
+     * window: slice s = 0 .. tq1 - tq0 + nj - 2 is frame t0 + K + j0 + nj - 1 - tq0 - s (ascending ring
+     * slots), which segment j reads for partition tq0 + s - (nj - 1 - j).  Shared memory holds NS
+     * buffers of QT G slices, then a circular window of NW = NS QT + nj - 1 slices (slice s in slot
+     * s % NW).  Tail stage k copies its G slices and only the window slices k QT + nj - 1 ..
+     * (k + 1) QT + nj - 2 (stage 0 also the first nj - 1): each ring slice is copied once.  Those
+     * overwrite slices (k - NS) QT .., which stage k - NS was the last to read -- and stage k is issued
+     * after every thread has passed stage k - NS. */
+    uint32_t tq0 = 0, tq1 = 0, n_titer = 0, QT = 1, NW = 1, Wg = 0, Wc4 = 1, nj = 1, boff = 0, slot_w0 = 0;
     if (LK != 0)
     {
         const uint32_t W    = M / LK;
         Wg                  = min(W, TB);
         Wc4                 = Wg / 2;
         nj                  = max(1u, TB / W);
-        j0                  = (tile * TB) / W;
-        p0                  = (tile * TB) % W;
-        QT                  = max(1u, ((2u * stage_elems) / Wg - (nj - 1)) / 2);
+        const uint32_t j0   = (tile * TB) / W;
+        boff                = a.la_c * W + (tile * TB) % W;                 /* bin offset of the slices */
+        QT                  = ((2u * NS * stage_elems) / Wg - (nj - 1)) / (2u * NS);
+        NW                  = NS * QT + nj - 1;
         uint32_t e0, e1;
         chunk_range(qe - qs, split, a.splits, sh.bias, e0, e1);
         tq0                 = qs + e0;
         tq1                 = qs + e1;
         n_titer             = (tq1 - tq0 + QT - 1) / QT;
+        /* window slice s is frame fmax - s, fmax = t0 + K + j0 + nj - 1 - tq0, in ring slot
+         * (slot0 + t - fmax + s) mod S (t - fmax >= 1 when the CTA has a tail) */
+        if (n_titer > 0)
+            slot_w0             = uint32_t((uint64_t(job.slot0) + (a.la_c + tq0 + 1u - (LK + j0 + nj))) % d.S);
     }
     const uint32_t t0       = job.tlo - a.la_c;                    /* first block of this launch's group */
 
@@ -2417,19 +2440,21 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
                 wait_ge<false>(a.ring_head + job.inst, t0, a.error, SPIN_ERR_RING);
                 asm volatile("fence.proxy.async;" ::: "memory");
             }
-            const uint32_t nx   = rows + nj - 1;
+            /* new window slices s0 .. s0 + nx - 1 */
+            const uint32_t s0   = (t_issued == 0) ? 0u : t_issued * QT + nj - 1;
+            const uint32_t nx   = rows + ((t_issued == 0) ? nj - 1 : 0u);
             const uint32_t sb   = Wg * uint32_t(sizeof(float2));
-            float2 *g           = stages + size_t(f_s) * 2 * stage_elems;
-            float2 *x           = g + size_t(QT) * Wg;
-            const uint64_t boff = uint64_t(a.la_c) * (M / LK) + p0;
+            float2 *g           = stages + size_t(f_s) * QT * Wg;
+            float2 *xw          = stages + size_t(NS) * QT * Wg;
             mbar_expect_tx(&full[f_s], (rows + nx) * sb);
             for (uint32_t r = 0; r < rows; ++r)
-                bulk_g2s(g + size_t(r) * Wg, d.G + uint64_t(q + r - d.q_lo) * M + boff, sb, &full[f_s], l2_stream);
-            /* frame fmax = t0 + K + j0 + nj - 1 - q lives in slot (slot0 + t - fmax) mod S, t - fmax >= 1 */
-            uint32_t sl         = uint32_t((uint64_t(job.slot0) + (a.la_c + q + 1u - (LK + j0 + nj))) % d.S);
+                bulk_g2s(g + size_t(r) * Wg, d.G + uint64_t(q + r - d.q_lo) * M + boff, sb, &full[f_s], stream_policy());
+            uint32_t ws         = s0 % NW;
+            uint32_t sl         = (slot_w0 + s0) % d.S;
             for (uint32_t i = 0; i < nx; ++i)
             {
-                bulk_g2s(x + size_t(i) * Wg, d.ring + uint64_t(sl) * M + boff, sb, &full[f_s], l2_stream);
+                bulk_g2s(xw + size_t(ws) * Wg, d.ring + uint64_t(sl) * M + boff, sb, &full[f_s], stream_policy());
+                if (++ws == NW)     ws = 0;
                 if (++sl == d.S)    sl = 0;
             }
             ++t_issued;
@@ -2463,6 +2488,9 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         uint32_t rows   = min(QB, q1 - q);
         float2 *g       = stages + size_t(f_s) * 2 * stage_elems;
         float2 *x       = g + stage_elems;
+        /* (an L2 policy is one instruction: made here rather than held in registers across the loops)
+         * the head rows of a lookahead launch are read again by the next 2K - 1 launches: keep them in L2 */
+        const uint64_t l2_head = (LK != 0) ? keep_policy() : stream_policy();
         mbar_expect_tx(&full[f_s], 2u * rows * row_bytes);
         bulk_g2s(g, Gt + uint64_t(q - d.q_lo) * M, rows * row_bytes, &full[f_s], l2_head);
         uint32_t n1     = min(rows, d.S - f_slot);
@@ -2475,8 +2503,9 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         if (f_slot >= d.S)  f_slot -= d.S;
     };
 
+    /* the head stages use the stage buffers that the tail's window covers: they follow the tail */
     if (tid == 0)
-        while ((t_issued + issued < NS) && (t_issued + issued < n_titer + n_main))
+        while ((t_issued + issued < NS) && (t_issued + issued < ((n_titer > 0) ? n_titer : n_main)))
             issue_next();
 
     float *po               = nullptr;
@@ -2585,52 +2614,62 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
 
     if (LK != 0)
     {
-        /* the lookahead tail: virtual columns lc = tid + v T of this tile, see above */
-        uint32_t gofs[MAC_VPT], xofs[MAC_VPT];
-        float tdn[MAC_VPT];
-        #pragma unroll
-        for (int v = 0; v < MAC_VPT; ++v)
+        /* The lookahead tail.  With several segments per tile (nj >= 2) a thread owns one float4 column
+         * and the two segments jv, jv + 1: segment jv + 1 multiplies partition q by the window slice that
+         * segment jv multiplied partition q - 1 by, so it comes from a register, and a partition costs the
+         * thread one G and one X load for both.  A tile inside one segment (nj = 1): columns tid and
+         * tid + T.  Every output still sums its partitions in ascending order, one fmaf chain each. */
+        const bool run      = (nj > 1);
+        const uint32_t col  = run ? tid % Wc4 : tid;
+        const uint32_t jv0  = run ? 2u * (tid / Wc4) : 0u;
+        float tdn[MAC_VPT]  = { 0.0f, 0.0f };
+        auto tail = [&](auto run_c)
         {
-            const uint32_t lc   = tid + v * T;
-            gofs[v]             = lc % Wc4;
-            xofs[v]             = (nj - 1 - lc / Wc4) * Wc4 + gofs[v];
-            tdn[v]              = 0.0f;
-        }
-        uint32_t t_cons = 0;
-        for (uint32_t it = 0; it < n_titer; ++it)
-        {
-            const uint32_t rows = min(QT, tq1 - (tq0 + t_cons * QT));
-            mbar_wait(&full[c_s], c_par);
-            const float4 *g4 = reinterpret_cast<const float4 *>(stages + size_t(c_s) * 2 * stage_elems);
-            const float4 *x4 = g4 + QT * Wc4;
-            for (uint32_t r = 0; r < rows; ++r)
+            constexpr bool RUN  = decltype(run_c)::value;
+            uint32_t xs         = nj - 1 - jv0;     /* window slot of segment jv0's operand for the next partition */
+            float4 xp           = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            const float4 *xw    = reinterpret_cast<const float4 *>(stages + size_t(NS) * QT * Wg);
+            for (uint32_t it = 0; it < n_titer; ++it)
             {
-                #pragma unroll
-                for (int v = 0; v < MAC_VPT; ++v)
+                const uint32_t rows = min(QT, tq1 - (tq0 + it * QT));
+                mbar_wait(&full[c_s], c_par);
+                const float4 *g4 = reinterpret_cast<const float4 *>(stages + size_t(c_s) * QT * Wg);
+                if (RUN && (it == 0))
+                    xp              = xw[(xs - 1) * Wc4 + col];
+                #pragma unroll 2
+                for (uint32_t r = 0; r < rows; ++r)
                 {
-                    float4 g    = g4[r * Wc4 + gofs[v]];
-                    float4 x    = x4[r * Wc4 + xofs[v]];
-                    acc[v].x    = fmaf(g.x, x.x, acc[v].x);
-                    acc[v].y    = fmaf(g.x, x.y, acc[v].y);
-                    acc[v].z    = fmaf(g.z, x.z, acc[v].z);
-                    acc[v].w    = fmaf(g.z, x.w, acc[v].w);
-                    acc[v].x    = fmaf(-g.y, x.y, acc[v].x);
-                    acc[v].y    = fmaf(g.y, x.x, acc[v].y);
-                    acc[v].z    = fmaf(-g.w, x.w, acc[v].z);
-                    acc[v].w    = fmaf(g.w, x.z, acc[v].w);
-                    tdn[v]      = fmaf(g.y, x.y, tdn[v]);
+                    const float4 g  = g4[r * Wc4 + col];
+                    const float4 x  = xw[xs * Wc4 + col];
+                    cmac(acc[0], tdn[0], g, x);
+                    if constexpr (RUN)
+                    {
+                        cmac(acc[1], tdn[1], g, xp);
+                        xp              = x;
+                    }
+                    else
+                        cmac(acc[1], tdn[1], g4[r * Wc4 + col + T], xw[xs * Wc4 + col + T]);
+                    if (++xs == NW) xs = 0;
                 }
+                if (++c_s == NS)    { c_s = 0; c_par ^= 1u; }
+                __syncthreads();
+                if ((tid == 0) && (t_issued < n_titer))
+                    issue_next();
             }
-            ++t_cons;
-            if (++c_s == NS)        { c_s = 0; c_par ^= 1u; }
-            __syncthreads();
-            if ((tid == 0) && ((t_issued < n_titer) || (issued < n_main)))
+        };
+        if (run)
+            tail(std::true_type());
+        else
+            tail(std::false_type());
+        /* every thread is past the last tail stage: the head stages may take the stage buffers */
+        if (tid == 0)
+            while ((issued < NS) && (issued < n_main))
                 issue_next();
-        }
+        FRAME_STAMP(4);
         /* bin 0 (DC, Nyquist) of the spectrum opens slice 0 of every segment */
         #pragma unroll
         for (int v = 0; v < MAC_VPT; ++v)
-            if ((a.la_c == 0) && (p0 == 0) && (gofs[v] == 0))
+            if ((boff == 0) && (col + (run ? 0u : v * T) == 0))
             {
                 acc[v].x       += tdn[v];
                 acc[v].y        = tdn[v];
@@ -2639,13 +2678,13 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         if (tid == 0)
             wait_ge<false>(a.la_cons + size_t(a.la_put) * a.n_cap + job.inst, a.la_put_need, a.error, SPIN_ERR_RING);
         __syncthreads();
-        float2 *tb      = a.la_T + uint64_t(a.la_put) * a.n_jobs * LK * a.splits * M
-                                 + uint64_t(a.la_c) * (M / LK) + p0;
+        float2 *tb      = a.la_T + uint64_t(a.la_put) * a.n_jobs * LK * a.splits * M + boff;
         #pragma unroll
         for (int v = 0; v < MAC_VPT; ++v)
         {
-            const uint32_t j    = j0 + (tid + v * T) / Wc4;
-            float4 *tp          = reinterpret_cast<float4 *>(tb + ((uint64_t(jobi) * LK + j) * a.splits + split) * M) + gofs[v];
+            const uint32_t j    = (tile * TB) / (M / LK) + jv0 + (run ? v : 0u);
+            float4 *tp          = reinterpret_cast<float4 *>(tb + ((uint64_t(jobi) * LK + j) * a.splits + split) * M)
+                                  + col + (run ? 0u : v * T);
             __stcg(tp, acc[v]);
             acc[v]              = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
@@ -2654,6 +2693,7 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
         if (tid == 0)
             asm volatile("red.release.gpu.global.add.u32 [%0], 1;"
                          :: "l"(a.la_prod + size_t(a.la_put) * a.n_cap + job.inst) : "memory");
+        FRAME_STAMP(5);
     }
 
     for (uint32_t it = 0; it < n_main; ++it)
@@ -2666,6 +2706,8 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
 
     if (GEN)
         FRAME_STAMP(5);
+    else if (LK != 0)
+        FRAME_STAMP(6);
     if (split0)
     {
         if (fft_cta)
@@ -2841,6 +2883,7 @@ __device__ __forceinline__ void frame_body(const StepArgs &a, const MacShape &sh
             __syncthreads();
             yT                  = a.la_T + ((uint64_t(a.la_get) * a.n_jobs + jobi) * LK + a.la_c) * a.splits * M;
             nT                  = a.splits;
+            FRAME_STAMP(7);
         }
         inv_body<RANK, TAIL_PP, TAIL_RG, int(T)>(wa, wb, ysum, nsum, job.dst, a.tw, tw, false, int(tid),
                                                  -1, nullptr, nullptr, yT, nT);
