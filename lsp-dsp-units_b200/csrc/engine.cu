@@ -331,22 +331,8 @@ static cudaError_t launch_mac_raw(const StepArgs &a, const MacPlan &p, uint32_t 
         attr_smem[dev] = p.smem;
     }
     dim3 grid(jobs * p.splits, p.tiles);
-    if (pdl)
-    {
-        /* may start while the preceding k_frame launch is in its tail (STEP_WAIT_HEAD) */
-        cudaLaunchConfig_t cfg;
-        memset(&cfg, 0, sizeof(cfg));
-        cfg.gridDim             = grid;
-        cfg.blockDim            = dim3(p.threads);
-        cfg.dynamicSmemBytes    = p.smem;
-        cfg.stream              = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id              = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs               = attr;
-        cfg.numAttrs            = 1;
-        return cudaLaunchKernelEx(&cfg, k_mac, a, p.sh);
-    }
+    if (pdl)            /* may start while the launch before it is in its tail (STEP_WAIT_HEAD, STEP_AFTER_FWD) */
+        return launch_k(k_mac, grid, dim3(p.threads), p.smem, st, true, a, p.sh);
     k_mac<<<grid, p.threads, p.smem, st>>>(a, p.sh);
     return cudaGetLastError();
 }
@@ -393,18 +379,7 @@ static cudaError_t launch_frame_r(const StepArgs &a, const MacPlan &p, uint32_t 
             return e;
         attr_smem[dev] = p.smem;
     }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim             = dim3(jobs * p.splits, p.tiles);
-    cfg.blockDim            = dim3(p.threads);
-    cfg.dynamicSmemBytes    = p.smem;
-    cfg.stream              = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id              = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
-    cfg.attrs               = attr;
-    cfg.numAttrs            = 1;
-    return cudaLaunchKernelEx(&cfg, k_frame<RANK>, a, p.sh, tickets, ra);
+    return launch_k(k_frame<RANK>, dim3(jobs * p.splits, p.tiles), dim3(p.threads), p.smem, st, pdl, a, p.sh, tickets, ra);
 }
 
 /* the job-list form (general path): no cross-GPU reduce; with `pdl` its prologue (and the launch
@@ -663,6 +638,30 @@ static const uint64_t LA_MIN_BYTES = 64000000ull;      /* k_frame lookahead: onl
                                                            would only pay for the extra T rows in their tail */
 static const size_t PART_MAX   = 1024;                  /* samples one P1 / P2 segment of a fused step answers */
 
+/* The launch schedules that reach from one process call into the next (DESIGN.md §4.1c, §5).  A
+ * launch that does not continue a schedule ends it: every launch path names the schedules it
+ * continues (SCHED_*) in one call of sched_continue, which ends all the others. */
+enum : uint32_t { SCHED_NONE = 0, SCHED_PEND = 1, SCHED_AHEAD = 2, SCHED_CHAIN = 4, SCHED_LA = 8 };
+struct Schedules
+{
+    /* eager pending MAC of synchronous callers: the rows of block t, for k_frame launch seq;
+     * last_was_frame: the last launch on the stream was a k_frame of this batch */
+    struct { bool ready = false; uint64_t t = 0; uint32_t splits = 0, seq = 0; bool last_was_frame = false; } pend;
+    /* ranks 14..16, the MAC one block ahead: partitions q >= 1 of block t are (being) summed into its row slot */
+    struct { bool valid = false; uint64_t t = 0; uint32_t splits = 0; } ahead;
+    /* three-kernel blocks: the chain-head word will hold `next` once everything enqueued has run */
+    struct { bool valid = false; uint32_t next = 0; } chain;
+    /* k_frame lookahead: the last launch of this batch was one; origin: batch frame of the schedule's
+     * priming group, next_t: the frame the next launch must carry to continue it.  The counters mirror
+     * d_la_cnt once everything enqueued has run (the same for every active instance): they outlive a
+     * schedule and are zeroed only with the device words (upload_tables). */
+    struct { bool live = false; uint32_t K = 0, splits = 0, nact = 0; uint64_t origin = 0, next_t = 0;
+             uint32_t prod_cnt[LA_BUFS] = { 0 }, cons_cnt[LA_BUFS] = { 0 }; } la;
+};
+
+/* How process_rows was called: from a synchronous host entry point; on page-locked host matrices */
+enum : uint32_t { CALL_SYNC = 1, CALL_HOST_IO = 2 };
+
 struct b200conv_batch
 {
     int                     device      = 0;
@@ -712,8 +711,7 @@ struct b200conv_batch
     int                     tune_splits = 0, tune_stages = 0;
     float                  *park        = nullptr;  /* k_inv_half scratch */
     size_t                  park_bytes  = 0;
-    bool                    last_was_frame = false; /* the last launch on the stream was a k_frame of this batch */
-    bool                    host_io     = false;    /* the running call reads / writes page-locked host matrices */
+    Schedules               sched;
     int                     opt_fused   = 1, opt_bias = 6, opt_pdl = 1, opt_zero_copy = 1, opt_multi = 8;
     int                     opt_early_src = 1;      /* 0 never, 1 on the batch's own stream, 2 on any stream */
     uint32_t               *d_tickets   = nullptr;  /* k_frame: [FRAME_SLOTS][instances] arrival counters */
@@ -722,24 +720,13 @@ struct b200conv_batch
     size_t                  ypart_slot_bytes = 0;   /* ypart holds FRAME_SLOTS slots of this size */
     std::vector<uint32_t>   h_slot_done;
     uint32_t               *d_ring_head = nullptr;  /* k_frame: frames published per instance; [n] = chain head (StepArgs::chain_head) */
-    bool                    chain_valid = false;    /* the device word will hold chain_next once everything enqueued has run */
-    uint32_t                chain_next  = 0;
     int                     opt_chain_ahead = 1;    /* ranks 14..16: the MAC of the NEXT block is launched behind this block's inverse transform */
-    bool                    ahead_valid = false;    /* partitions q >= 1 of block ahead_t are (being) summed into its row slot */
-    uint64_t                ahead_t     = 0;
-    uint32_t                ahead_splits = 0;
     uint32_t               *h_error     = nullptr;  /* page-locked, device-mapped: a bounded in-kernel wait gave up */
     /* k_frame lookahead for one-frame calls (kernels.cuh, LA_BUFS) */
     int                     opt_lookahead = -1;     /* -1 automatic, 0 off, 2 / 4 / 8 = that group size K */
     float2                 *la_T        = nullptr;  /* [LA_BUFS][jobs][K][splits][M] */
     size_t                  la_T_bytes  = 0;
     uint32_t               *d_la_cnt    = nullptr;  /* [2][LA_BUFS][instances]: producer CTAs, consumer tails */
-    bool                    la_live     = false;    /* the last launch of this batch was a lookahead k_frame (la_* below) */
-    uint32_t                la_K        = 0, la_splits = 0, la_nact = 0;
-    uint64_t                la_origin   = 0;        /* batch frame of the first block of the schedule (priming group) */
-    uint64_t                la_next_t   = 0;        /* batch frame the next launch must carry to continue it */
-    uint32_t                la_prod_cnt[LA_BUFS] = { 0 }, la_cons_cnt[LA_BUFS] = { 0 };    /* the device counters once
-                                                       everything enqueued has run (same for every active instance) */
     std::vector<uint32_t>   h_ring_head;
 
     /* eager pending MAC for synchronous host callers: right after block t has been delivered the
@@ -748,11 +735,6 @@ struct b200conv_batch
     int                     opt_eager   = 1;
     int                     opt_early_pend = 1;     /* the pending MAC may start under the tail of the launch before it: 0 never, 1 auto, 2 always */
     bool                    caller_busy = false;    /* the previous pending MAC was still running when the current call arrived */
-    bool                    eager_call  = false;    /* set by the synchronous entry points */
-    bool                    pend_ready  = false;
-    uint64_t                pend_t      = 0;        /* batch frame counter the pending rows belong to */
-    uint32_t                pend_splits = 0;
-    uint32_t                pend_seq    = 0;        /* sequence number of the k_frame launch the pending rows are for */
     cudaEvent_t             ev_done     = nullptr;  /* output of the current block is complete */
     cudaEvent_t             ev_pend     = nullptr;  /* the pending MAC launched after it is complete */
     bool                    pend_inflight = false;
@@ -770,22 +752,22 @@ struct b200conv_batch
 
 typedef b200conv_batch Batch;
 
-static cudaError_t launch_mac(Batch *b, const StepArgs &a, const MacPlan &p, uint32_t jobs, cudaStream_t st,
-                              bool fused = false, bool serial = false, bool chain = false)
+/* Ends every schedule that `keep` (SCHED_*) does not name.  Each launch path calls it once, after
+ * it has read the state of the schedules it continues; so do the calls that make a schedule's
+ * state meaningless (new tables, buffers or options). */
+static void sched_continue(Batch *b, uint32_t keep)
 {
-    auto go = [&]() -> cudaError_t
-    {
-        if (fused)
-        {
-            const uint32_t slot = a.seq % uint32_t(FRAME_SLOTS);
-            ReduceArgs ra   = b->reduce;
-            if (ra.mode != 0)
-                ra.scratch     += size_t(slot) * ra.channels * ra.frame;
-            return launch_frame(a, p, jobs, b->d_tickets + size_t(slot) * b->n, ra,
-                                (b->opt_pdl != 0) && (!b->profiling) && (!serial), st);
-        }
-        return launch_mac_raw(a, p, jobs, st, chain);
-    };
+    Schedules &s = b->sched;
+    if (!(keep & SCHED_PEND))   s.pend.ready = s.pend.last_was_frame = false;
+    if (!(keep & SCHED_AHEAD))  s.ahead.valid = false;
+    if (!(keep & SCHED_CHAIN))  s.chain.valid = false;
+    if (!(keep & SCHED_LA))     s.la.live = false;
+}
+
+/* Runs `go` (one MAC launch) between the two events b200conv_get_profile reads, when profiling. */
+template <typename Launch>
+static cudaError_t profiled(Batch *b, cudaStream_t st, Launch go)
+{
     if (!b->profiling)
         return go();
     while (b->prof_events.size() < b->prof_used + 2)
@@ -801,6 +783,23 @@ static cudaError_t launch_mac(Batch *b, const StepArgs &a, const MacPlan &p, uin
     if (e == cudaSuccess) e = cudaEventRecord(b->prof_events[b->prof_used + 1], st);
     b->prof_used += 2;
     return e;
+}
+
+/* One k_frame launch of the uniform path; `serial`: without programmatic serialisation */
+static cudaError_t launch_kframe(Batch *b, const StepArgs &a, const MacPlan &p, uint32_t jobs, cudaStream_t st, bool serial)
+{
+    const uint32_t slot = a.seq % uint32_t(FRAME_SLOTS);
+    ReduceArgs ra   = b->reduce;
+    if (ra.mode != 0)
+        ra.scratch     += size_t(slot) * ra.channels * ra.frame;
+    const bool pdl  = (b->opt_pdl != 0) && (!b->profiling) && (!serial);
+    return profiled(b, st, [&]() { return launch_frame(a, p, jobs, b->d_tickets + size_t(slot) * b->n, ra, pdl, st); });
+}
+
+/* One k_mac launch; `pdl`: with programmatic serialisation */
+static cudaError_t launch_kmac(Batch *b, const StepArgs &a, const MacPlan &p, uint32_t jobs, cudaStream_t st, bool pdl)
+{
+    return profiled(b, st, [&]() { return launch_mac_raw(a, p, jobs, st, pdl); });
 }
 
 /* Makes the batch's device current for the duration of an API call and restores the caller's
@@ -904,7 +903,7 @@ static void rebuild_tables(Batch *b)
         d.S         = uint32_t(in.S);
     }
     b->desc_dirty = true;
-    b->pend_ready = false;
+    sched_continue(b, SCHED_NONE);
 }
 
 static int upload_tables(Batch *b, cudaStream_t st)
@@ -912,8 +911,7 @@ static int upload_tables(Batch *b, cudaStream_t st)
     if (!b->desc_dirty)
         return B200CONV_OK;
     hist_reset(st, b->device);          /* the copies below are full dependencies */
-    b->chain_valid = false;
-    b->ahead_valid = false;
+    sched_continue(b, SCHED_NONE);
     for (size_t i = 0; i < b->n; ++i)
     {
         b->h_ring_head[i]   = uint32_t(b->inst[i].frames);
@@ -928,8 +926,7 @@ static int upload_tables(Batch *b, cudaStream_t st)
     /* ... and no lookahead tail is pending: the schedule restarts with a priming group */
     CU(cudaMemsetAsync(b->d_la_cnt, 0, 2 * LA_BUFS * b->n * sizeof(uint32_t), st));
     for (int i = 0; i < LA_BUFS; ++i)
-        b->la_prod_cnt[i] = b->la_cons_cnt[i] = 0;
-    b->la_live          = false;
+        b->sched.la.prod_cnt[i] = b->sched.la.cons_cnt[i] = 0;
     /* pageable sources: cudaMemcpyAsync stages them before returning */
     CU(cudaMemcpyAsync(b->d_desc, b->h_desc.data(), b->n * sizeof(InstDesc), cudaMemcpyHostToDevice, st));
     if (!b->active.empty())
@@ -956,7 +953,10 @@ static int ensure_ypart(Batch *b, size_t bytes, cudaStream_t st)
     CU(cudaMalloc(&b->ypart, want * FRAME_SLOTS));
     b->ypart_bytes  = want * FRAME_SLOTS;
     b->ypart_slot_bytes = want;
-    b->pend_ready   = false;
+    /* the pending and ahead rows were in the old buffer; the chain-head word is not, so the chain
+     * goes on (ending it would cost a seeding copy when another batch's "mac_tile" grows this
+     * batch's splits between two chained blocks) */
+    sched_continue(b, SCHED_CHAIN);
     return B200CONV_OK;
 }
 
@@ -971,7 +971,7 @@ static int ensure_la(Batch *b, size_t bytes, cudaStream_t st)
         cudaFree(b->la_T);
     b->la_T         = nullptr;
     b->la_T_bytes   = 0;
-    b->la_live      = false;
+    sched_continue(b, SCHED_NONE);
     CU(cudaMalloc(&b->la_T, bytes));
     b->la_T_bytes   = bytes;
     return B200CONV_OK;
@@ -1076,14 +1076,14 @@ static int push_jobs(Batch *b, size_t pos, size_t count, cudaStream_t st)
     return B200CONV_OK;
 }
 
-static StepArgs base_args(const Batch *b)
+static StepArgs base_args(const Batch *b, uint32_t mode)
 {
     StepArgs a;
     memset(&a, 0, sizeof(a));
     a.inst      = b->d_desc;
     a.active    = b->d_active;
     a.tw        = b->tw[b->rank];
-    a.flags     = b->host_io ? uint32_t(STEP_HOST_IO) : 0u;
+    a.flags     = (mode & CALL_HOST_IO) ? uint32_t(STEP_HOST_IO) : 0u;
     a.ypart     = b->ypart;
     a.ring_head = b->d_ring_head;
     a.error     = b->h_error;       /* UVA: the mapped host word is addressable from the device */
@@ -1496,7 +1496,7 @@ static int init_many_impl(b200conv_batch_t *b, size_t count, const size_t *idx, 
 
             /* H_p = spectrum of taps [pF, (p+1)F) zero padded -- the per-partition fastconv_parse of
              * Convolver.cpp:183-197 for every partition of every instance of the round, one launch */
-            StepArgs a  = base_args(b);
+            StepArgs a  = base_args(b, 0);
             a.rank      = uint32_t(rank);
             a.tw        = b->tw[rank];
             a.jobs      = nullptr;
@@ -1640,289 +1640,311 @@ static int init_shared_impl(b200conv_batch_t *b, size_t idx, size_t src_idx, flo
 /* ------------------------------------------------------------------------------------------- */
 /* process                                                                                      */
 
-/* All active instances sit on a frame boundary and `frames` whole frames arrive: derive the
- * jobs on the device, three launches per frame for all instances x partitions. */
 static bool eager_possible(const Batch *b)
 {
     return (b->opt_eager != 0) && (b->opt_fused != 0) && (b->rank >= 8) && (b->rank <= 11) &&
            (b->reduce.mode == 0) && (!b->profiling) && (!b->active.empty());
 }
 
-static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float *src, size_t stride,
-                           size_t frames, cudaStream_t st)
+/* One process_uniform call, as its step functions (step_*) see it; `a` is carried from one step to
+ * the next.  A step returns the frames it consumed, or a (negative) error code. */
+struct UniformCall
 {
-    const uint32_t nact = uint32_t(b->active.size());
+    StepArgs        a;
+    MacPlan         plan;
+    size_t          F, frames;
+    uint32_t        nact, mode;
+    uint64_t        per_frame_bytes;    /* algorithmic MAC bytes of one block */
+    bool            tables_changed;     /* the call uploaded new tables */
+    cudaStream_t    st;
+};
+
+/* Stats of one step: `launches` kernels and one MAC pass for `frames` blocks */
+static void count_step(Batch *b, const UniformCall &c, uint32_t launches, uint32_t frames, uint64_t stream_bytes)
+{
+    b->stats.launches           += launches;
+    b->stats.mac_launches       += 1;
+    b->stats.mac_algo_bytes     += c.per_frame_bytes * frames;
+    b->stats.mac_stream_bytes   += stream_bytes;
+    b->stats.frames             += uint64_t(c.nact) * frames;
+}
+
+/* Registers the launch that reads input block f and writes output block f with the launch
+ * history of the stream (FrameHistory, hist_launch). */
+static void block_history(const Batch *b, const UniformCall &c, size_t f, bool capable,
+                          bool *early, bool *serial, bool *dst_clash)
+{
+    const size_t F      = c.F;
+    const BlockRows in  = { reinterpret_cast<uintptr_t>(c.a.src + f * F), c.a.stride * sizeof(float), F * sizeof(float), b->n };
+    const BlockRows out = { reinterpret_cast<uintptr_t>(c.a.dst + f * F), c.a.stride_dst * sizeof(float), F * sizeof(float), b->n };
+    hist_launch(c.st, b->device, capable, in, out, early, serial, dst_clash);
+}
+
+/* Several whole frames in one call: transform them all, then ONE pass over the IR spectra serves
+ * tf frames (k_mac_multi), then all inverse transforms. */
+static int step_multi(Batch *b, UniformCall &c, uint32_t tf)
+{
+    StepArgs &a     = c.a;
+    MacPlan mp      = c.plan;
+    mp.sh.bias      = 0;
+    /* the register window limits occupancy (8 frames: 1 CTA/SM, 4: 2, 2: 3), so the
+     * bytes in flight come from a deeper shared-memory ring instead */
+    mp.sh.NS        = (tf == 8) ? 8 : (tf == 4) ? 6 : 4;
+    mp.smem         = size_t(2) * mp.sh.NS * mp.sh.QB * mp.sh.TB * sizeof(float2) + 2 * mp.sh.NS * sizeof(uint64_t) + 16;
+    TRY(ensure_ypart(b, size_t(c.nact) * tf * mp.splits * c.F * sizeof(float2), c.st));
+    hist_reset(c.st, b->device);
+    a.ypart         = b->ypart;
+    a.n_jobs        = c.nact * tf;
+    CU(launch_fwd(a, c.nact * tf, c.st));
+    CU(launch_mac_multi(a, mp, c.nact, tf, c.st));
+    TRY(attach_park(b, a, size_t(c.nact) * tf, c.st));
+    CU(launch_inv(a, c.nact * tf, c.st));
+    hist_unknown(c.st, b->device);
+    sched_continue(b, SCHED_NONE);
+    count_step(b, c, 3, tf, c.per_frame_bytes * tf);
+    return int(tf);
+}
+
+/* Block f in one k_frame launch for all instances x partitions (ranks 8..13): in a stream of
+ * one-frame calls with the lookahead, and after the pending MAC of a synchronous caller as the
+ * head-only launch that consumes it. */
+static int step_frame(Batch *b, UniformCall &c, size_t f)
+{
+    Schedules &s    = b->sched;
+    StepArgs &a     = c.a;
+    const MacPlan &plan = c.plan;
+    /* Lookahead (kernels.cuh, LA_BUFS): a stream of one-frame calls in uniform mode.  Chosen from
+     * the call pattern and the batch's shape only -- never from pdl, profiling, the stream or the
+     * early-read options -- so that every way of running a stream sums in the same order.  A
+     * synchronous call, a multi-frame call, the general path or any table change ends the schedule;
+     * the next one starts with a priming group (full sums, tails for the group after it). */
+    uint32_t K      = 0;
+    if ((c.frames == 1) && !(c.mode & CALL_SYNC) && (b->reduce.mode == 0))
+        K               = lookahead_k(b, c.per_frame_bytes);
+    uint64_t launch_bytes = c.per_frame_bytes;
+    a.la_K          = 0;
+    if (K != 0)
+    {
+        const uint64_t t    = a.t_base + f;
+        if ((!s.la.live) || (s.la.K != K) || (s.la.splits != plan.splits) || (s.la.nact != c.nact) ||
+            c.tables_changed || (s.la.next_t != t))
+        {
+            TRY(ensure_la(b, size_t(LA_BUFS) * c.nact * K * plan.splits * c.F * sizeof(float2), c.st));
+            s.la.origin     = t;
+        }
+        const uint64_t rel  = t - s.la.origin;
+        const uint32_t g    = uint32_t((rel / K) % LA_BUFS);
+        a.la_T          = b->la_T;
+        a.la_prod       = b->d_la_cnt;
+        a.la_cons       = b->d_la_cnt + LA_BUFS * b->n;
+        a.la_K          = K;
+        a.la_c          = uint32_t(rel % K);
+        a.la_use        = (rel >= K) ? 1u : 0u;
+        a.la_get        = g;
+        a.la_put        = (g + 1) % LA_BUFS;
+        a.la_put_need   = s.la.cons_cnt[a.la_put];
+        a.la_get_need   = s.la.prod_cnt[a.la_get];
+        if (a.la_use)
+            s.la.cons_cnt[a.la_get] += 1;
+        s.la.prod_cnt[a.la_put] += plan.splits * plan.tiles;
+        s.la.live       = true;
+        s.la.K          = K;
+        s.la.splits     = plan.splits;
+        s.la.nact       = c.nact;
+        s.la.next_t     = t + 1;
+        launch_bytes    = 0;
+        for (uint32_t i : b->active)
+            launch_bytes   += la_stream_bytes(b->inst[i], K, a.la_use != 0, plan.sh, plan.splits);
+    }
+    /* May its input transform run ahead of the launches still in flight on this stream?
+     * (FrameHistory) -- worth it only while the transform is a visible share of the block: a
+     * launch that streams for tens of microseconds hides the chain anyway */
+    bool early = false, serial = false, dst_clash = false;
+    const bool capable = (b->opt_pdl != 0) && (!b->profiling) && (launch_bytes <= EARLY_MAX_BYTES) &&
+                         ((b->opt_early_src == 2) || ((b->opt_early_src == 1) && (c.st == b->stream)));
+    block_history(b, c, f, capable, &early, &serial, &dst_clash);
+    a.flags        &= ~uint32_t(STEP_EARLY_SRC | STEP_ORDER_DST);
+    if (early)
+        a.flags        |= STEP_EARLY_SRC;
+    if (dst_clash)
+        a.flags        |= STEP_ORDER_DST;  /* e.g. a cascade re-using one hand-over block: the tail of the
+                                              next launch must not overwrite what a launch in flight reads */
+    /* pipelined tails (FRAME_SLOTS in kernels.cuh): this launch's rows, tickets and sequence number */
+    a.seq           = b->frame_seq;
+    a.n_cap         = uint32_t(b->n);
+    a.slot_done     = ((b->opt_pdl != 0) && (!b->profiling)) ? b->d_slot_done : nullptr;
+    a.ypart         = ypart_slot(b, a.seq);
+    if (a.slot_done != nullptr)
+        b->frame_seq   += 1;            /* only pipelined launches take part in the slot rotation */
+    const bool eager = (c.mode & CALL_SYNC) && (c.frames == 1) && eager_possible(b);
+    if (eager && s.pend.ready && (s.pend.t == a.t_base + f) && (s.pend.splits == plan.splits) &&
+        (!c.tables_changed) && (s.pend.seq == a.seq))
+    {
+        /* partitions q >= 1 were summed ahead of time (launch_pending_mac): transform the
+         * input, add partition 0, invert -- one CTA per instance */
+        MacPlan fp      = plan;
+        fp.splits       = 1;
+        fp.sh.bias      = 0;
+        StepArgs af     = a;
+        af.splits       = 1;
+        af.rows         = s.pend.splits + 1;
+        af.row0         = s.pend.splits;
+        af.sum0         = s.pend.splits - 1;        /* the pending MAC folded its rows into this one */
+        af.flags       |= STEP_HEAD_ONLY;
+        /* A synchronous host call on the own stream: every launch that delivered an earlier
+         * block has completed (the caller has its output), and the predecessor in the
+         * stream is this batch's pending MAC, which never touches the caller's input block
+         * -- the block is fetched and transformed under that MAC whatever the launch size. */
+        if ((c.st == b->stream) && (b->opt_pdl != 0) && (b->opt_early_src != 0))
+            af.flags       |= STEP_EARLY_SRC;
+        CU(launch_kframe(b, af, fp, c.nact, c.st, serial));
+    }
+    else
+        CU(launch_kframe(b, a, plan, c.nact, c.st, serial));
+    sched_continue(b, (K != 0) ? SCHED_LA : SCHED_NONE);
+    s.pend.last_was_frame = (c.st == b->stream) && (!b->profiling);
+    count_step(b, c, 1, 1, launch_bytes);
+    return 1;
+}
+
+/* Block f through k_fwd, k_mac and k_inv: ranks 14..16, and ranks 8..13 with fused = 0 or after a
+ * multi-frame pass of the same call. */
+static int step_three(Batch *b, UniformCall &c, size_t f)
+{
+    Schedules &s    = b->sched;
+    StepArgs &a     = c.a;
+    MacPlan sp      = c.plan;
+    sp.sh.bias      = 0;
+    const bool ahead = (b->rank >= 14) && (b->opt_pdl != 0) && (!b->profiling) && (b->opt_chain_ahead != 0) && (c.frames == 1);
+    if (ahead)
+    {
+        /* Block-by-block callers at ranks 14..16: partitions q >= 1 of block t need complete frames
+         * only, so their MAC is launched one block AHEAD -- behind the inverse transform of block
+         * t - 1 -- into a row slot of its own, and streams under that inverse transform and under
+         * the transform of block t; partition 0 is added by the inverse transform of block t
+         * (STEP_Q0_IN_INV).  Stream order per call:  k_fwd(t)  k_inv(t)  k_mac(t + 1).
+         * What orders them: chain_head ("frames < x are final", published by k_inv(t) once
+         * k_fwd(t) has completed; k_mac(t + 1) polls it), row slots t mod FRAME_SLOTS, and one
+         * CTA of every kernel that waits for the launch before it as its last instruction. */
+        const uint64_t t    = a.t_base + a.frame0;
+        const uint32_t t32  = uint32_t(t);
+        uint32_t *head      = b->d_ring_head + b->n;
+        auto mac_ahead = [&](uint64_t t_of, bool pdl) -> cudaError_t
+        {
+            StepArgs am     = a;
+            am.t_base       = t_of - a.frame0;
+            am.ypart        = ypart_slot(b, uint32_t(t_of));
+            am.flags       |= STEP_FROM_Q1 | STEP_AHEAD;
+            am.chain_head   = head;
+            return launch_kmac(b, am, sp, c.nact, c.st, pdl);
+        };
+        const bool cold = !(s.ahead.valid && (s.ahead.t == t) && (s.ahead.splits == sp.splits));
+        if (cold)
+        {
+            /* cold start (or a MAC launched ahead for a block that never came): seed the chain head by
+             * a copy and launch this block's MAC without the attribute -- both full dependencies */
+            CU(cudaMemcpyAsync(head, &t32, sizeof(t32), cudaMemcpyHostToDevice, c.st));
+            CU(mac_ahead(t, false));
+        }
+        bool early = false, serial = false, dst_clash = false;
+        block_history(b, c, f, (b->opt_early_src == 2) || ((b->opt_early_src == 1) && (c.st == b->stream)),
+                      &early, &serial, &dst_clash);
+        StepArgs ai     = a;
+        ai.ypart        = ypart_slot(b, t32);
+        TRY(attach_park(b, ai, c.nact, c.st));      /* (may synchronise) */
+        StepArgs af     = a;
+        if (early)
+            af.flags       |= STEP_EARLY_SRC;
+        CU(launch_fwd(af, c.nact, c.st, !serial));
+        ai.flags       |= STEP_Q0_IN_INV;
+        ai.chain_head   = head;
+        CU(launch_inv(ai, c.nact, c.st, true, b->d_tickets));
+        CU(mac_ahead(t + 1, true));
+        sched_continue(b, SCHED_AHEAD | SCHED_CHAIN);
+        s.ahead         = { true, t + 1, sp.splits };
+        s.chain         = { true, t32 + 1u };
+        count_step(b, c, cold ? 4 : 3, 1, c.per_frame_bytes);
+        return 1;
+    }
+    hist_reset(c.st, b->device);
+    /* Ranks 14..16: the three kernels of a block are chained with programmatic serialisation --
+     * the partition stream of q >= 1 runs beside the block's own transform (which only the
+     * stage with q = 0 needs, taken last, STEP_AFTER_FWD), table staging overlaps the launch
+     * before; every kernel orders itself with griddepcontrol.wait. */
+    const bool chain = (b->rank >= 14) && (b->opt_pdl != 0) && (!b->profiling);
+    TRY(attach_park(b, a, c.nact, c.st));       /* (may synchronise: before the chain starts) */
+    CU(launch_fwd(a, c.nact, c.st, chain));
+    StepArgs am     = a;
+    if (chain)
+        am.flags       |= STEP_AFTER_FWD;
+    /* "the spectra of all frames < t are final": published by the k_mac of block t - 1; whenever
+     * that was not the launch before this one (first block, a multi-frame pass, the general
+     * path, another frame counter) the word is seeded by a copy -- a full dependency */
+    const uint32_t t32 = uint32_t(a.t_base + a.frame0);
+    if ((!s.chain.valid) || (s.chain.next != t32))
+        CU(cudaMemcpyAsync(b->d_ring_head + b->n, &t32, sizeof(t32), cudaMemcpyHostToDevice, c.st));
+    am.chain_head   = b->d_ring_head + b->n;
+    sched_continue(b, SCHED_CHAIN);
+    s.chain         = { true, t32 + 1u };
+    CU(launch_kmac(b, am, sp, c.nact, c.st, chain));
+    CU(launch_inv(a, c.nact, c.st, chain, b->d_tickets));      /* nact <= instances counters */
+    hist_unknown(c.st, b->device);
+    count_step(b, c, 3, 1, c.per_frame_bytes);
+    return 1;
+}
+
+/* All active instances sit on a frame boundary and `frames` whole frames arrive: the kernels
+ * derive their jobs from the call (uniform mode), one step per block or per multi-frame pass. */
+static int process_uniform(Batch *b, float *dst, size_t dst_stride, const float *src, size_t stride,
+                           size_t frames, cudaStream_t st, uint32_t mode)
+{
+    UniformCall c;
+    c.nact          = uint32_t(b->active.size());
     if (b->uniform_stale)
         b->desc_dirty   = true;         /* the general path moved the frame counters one by one */
     b->uniform_stale = false;
-    const bool tables_changed = b->desc_dirty;
+    c.tables_changed = b->desc_dirty;
     TRY(upload_tables(b, st));
-    MacPlan plan    = plan_mac(uint32_t(b->rank), nact, uint32_t(b->max_nq), b->sm_count,
+    c.plan          = plan_mac(uint32_t(b->rank), c.nact, uint32_t(b->max_nq), b->sm_count,
                                b->tune_splits, b->tune_stages);
-    const size_t F  = size_t(1) << (b->rank - 1);
-    const bool eager = b->eager_call && (frames == 1) && eager_possible(b);
+    c.F             = size_t(1) << (b->rank - 1);
+    c.frames        = frames;
+    c.mode          = mode;
+    c.st            = st;
     /* one extra row per job when the pending MAC runs ahead (it must not be re-allocated between
      * the pending launch and the call that consumes it) */
-    TRY(ensure_ypart(b, size_t(nact) * (plan.splits + 1) * F * sizeof(float2), st));
-    if (tables_changed || (b->pend_splits != plan.splits))
-        b->pend_ready   = false;
+    TRY(ensure_ypart(b, size_t(c.nact) * (c.plan.splits + 1) * c.F * sizeof(float2), st));
 
-    uint64_t per_frame_bytes = 0;
+    c.per_frame_bytes = 0;
     for (uint32_t i : b->active)
-        per_frame_bytes += algo_bytes(b, b->inst[i], 0, size_t(-1));
+        c.per_frame_bytes += algo_bytes(b, b->inst[i], 0, size_t(-1));
 
-    StepArgs a      = base_args(b);
+    StepArgs &a     = c.a;
+    a               = base_args(b, mode);
     a.src           = src;
     a.dst           = dst;
     a.stride        = stride;
     a.stride_dst    = dst_stride;
-    a.splits        = plan.splits;
-    a.n_jobs        = nact;
+    a.splits        = c.plan.splits;
     a.t_base        = b->t_batch;
     const bool fused = (b->opt_fused != 0) && (b->rank <= 13);     /* k_frame: ranks 8..13 */
     if ((b->reduce.mode != 0) && (!fused))
         return fail(B200CONV_ERR_STATE, "the fused cross-GPU reduce needs the one-launch-per-block path (ranks 8..13, fused = 1)");
-    plan.sh.bias    = fused ? uint32_t(b->opt_bias) : 0;
+    c.plan.sh.bias  = fused ? uint32_t(b->opt_bias) : 0;
     bool used_multi = false;
     for (size_t f = 0; f < frames; )
     {
         a.frame0        = uint32_t(f);
-        a.n_jobs        = nact;
-        /* several whole frames in one call: transform them all, then ONE pass over the IR
-         * spectra serves tf frames (k_mac_multi), then all inverse transforms */
+        a.n_jobs        = c.nact;
         uint32_t tf     = 0;
-        for (uint32_t c = (b->reduce.mode != 0) ? 0u : uint32_t(b->opt_multi); c >= 2; c >>= 1)
-            if (frames - f >= c) { tf = c; break; }
-        if (tf >= 2)
-        {
-            MacPlan mp      = plan;
-            mp.sh.bias      = 0;
-            /* the register window limits occupancy (8 frames: 1 CTA/SM, 4: 2, 2: 3), so the
-             * bytes in flight come from a deeper shared-memory ring instead */
-            mp.sh.NS        = (tf == 8) ? 8 : (tf == 4) ? 6 : 4;
-            mp.smem         = size_t(2) * mp.sh.NS * mp.sh.QB * mp.sh.TB * sizeof(float2) + 2 * mp.sh.NS * sizeof(uint64_t) + 16;
-            TRY(ensure_ypart(b, size_t(nact) * tf * mp.splits * F * sizeof(float2), st));
-            hist_reset(st, b->device);
-            a.ypart         = b->ypart;
-            a.n_jobs        = nact * tf;
-            CU(launch_fwd(a, nact * tf, st));
-            CU(launch_mac_multi(a, mp, nact, tf, st));
-            TRY(attach_park(b, a, size_t(nact) * tf, st));
-            CU(launch_inv(a, nact * tf, st));
-            hist_unknown(st, b->device);
-            b->chain_valid  = false;
-            b->ahead_valid  = false;
-            b->la_live      = false;
-            b->stats.launches       += 3;
-            b->stats.mac_launches   += 1;
-            b->stats.mac_algo_bytes += per_frame_bytes * tf;
-            b->stats.mac_stream_bytes += per_frame_bytes * tf;
-            b->stats.frames         += uint64_t(nact) * tf;
-            used_multi      = true;
-            b->pend_ready   = false;
-            f              += tf;
-            continue;
-        }
-        if (fused && (!used_multi))
-        {
-            /* Lookahead (kernels.cuh, LA_BUFS): a stream of one-frame calls in uniform mode.  Chosen from
-             * the call pattern and the batch's shape only -- never from pdl, profiling, the stream or the
-             * early-read options -- so that every way of running a stream sums in the same order.  A
-             * synchronous call, a multi-frame call, the general path or any table change ends the schedule;
-             * the next one starts with a priming group (full sums, tails for the group after it). */
-            uint32_t K      = 0;
-            if ((frames == 1) && (!b->eager_call) && (b->reduce.mode == 0))
-                K               = lookahead_k(b, per_frame_bytes);
-            uint64_t launch_bytes = per_frame_bytes;
-            a.la_K          = 0;
-            if (K != 0)
-            {
-                const uint64_t t    = a.t_base + f;
-                if ((!b->la_live) || (b->la_K != K) || (b->la_splits != plan.splits) || (b->la_nact != nact) ||
-                    tables_changed || (b->la_next_t != t))
-                {
-                    TRY(ensure_la(b, size_t(LA_BUFS) * nact * K * plan.splits * F * sizeof(float2), st));
-                    b->la_origin    = t;
-                }
-                const uint64_t rel  = t - b->la_origin;
-                const uint32_t g    = uint32_t((rel / K) % LA_BUFS);
-                a.la_T          = b->la_T;
-                a.la_prod       = b->d_la_cnt;
-                a.la_cons       = b->d_la_cnt + LA_BUFS * b->n;
-                a.la_K          = K;
-                a.la_c          = uint32_t(rel % K);
-                a.la_use        = (rel >= K) ? 1u : 0u;
-                a.la_get        = g;
-                a.la_put        = (g + 1) % LA_BUFS;
-                a.la_put_need   = b->la_cons_cnt[a.la_put];
-                a.la_get_need   = b->la_prod_cnt[a.la_get];
-                if (a.la_use)
-                    b->la_cons_cnt[a.la_get] += 1;
-                b->la_prod_cnt[a.la_put] += plan.splits * plan.tiles;
-                b->la_live      = true;
-                b->la_K         = K;
-                b->la_splits    = plan.splits;
-                b->la_nact      = nact;
-                b->la_next_t    = t + 1;
-                launch_bytes    = 0;
-                for (uint32_t i : b->active)
-                    launch_bytes   += la_stream_bytes(b->inst[i], K, a.la_use != 0, plan.sh, plan.splits);
-            }
-            else
-                b->la_live      = false;
-            /* one launch per block for all instances x partitions.  May its input transform run
-             * ahead of the launches still in flight on this stream? (FrameHistory) */
-            bool early = false, serial = false, dst_clash = false;
-            {
-                /* worth it only while the transform is a visible share of the block: a launch that
-                 * streams for tens of microseconds hides the chain anyway */
-                const bool capable = (b->opt_pdl != 0) && (!b->profiling) && (launch_bytes <= EARLY_MAX_BYTES) &&
-                                     ((b->opt_early_src == 2) || ((b->opt_early_src == 1) && (st == b->stream)));
-                const BlockRows in  = { reinterpret_cast<uintptr_t>(src + f * F), stride * sizeof(float), F * sizeof(float), b->n };
-                const BlockRows out = { reinterpret_cast<uintptr_t>(dst + f * F), dst_stride * sizeof(float), F * sizeof(float), b->n };
-                hist_launch(st, b->device, capable, in, out, &early, &serial, &dst_clash);
-            }
-            a.flags        &= ~uint32_t(STEP_EARLY_SRC | STEP_ORDER_DST);
-            if (early)
-                a.flags        |= STEP_EARLY_SRC;
-            if (dst_clash)
-                a.flags        |= STEP_ORDER_DST;  /* e.g. a cascade re-using one hand-over block: the tail of the
-                                                      next launch must not overwrite what a launch in flight reads */
-            /* pipelined tails (FRAME_SLOTS in kernels.cuh): this launch's rows, tickets and sequence number */
-            a.seq           = b->frame_seq;
-            a.n_cap         = uint32_t(b->n);
-            a.slot_done     = ((b->opt_pdl != 0) && (!b->profiling)) ? b->d_slot_done : nullptr;
-            a.ypart         = ypart_slot(b, a.seq);
-            if (a.slot_done != nullptr)
-                b->frame_seq   += 1;            /* only pipelined launches take part in the slot rotation */
-            if (eager && b->pend_ready && (b->pend_t == b->t_batch + f) && (!tables_changed) && (b->pend_seq == a.seq))
-            {
-                /* partitions q >= 1 were summed ahead of time (launch_pending_mac): transform the
-                 * input, add partition 0, invert -- one CTA per instance */
-                MacPlan fp      = plan;
-                fp.splits       = 1;
-                fp.sh.bias      = 0;
-                StepArgs af     = a;
-                af.splits       = 1;
-                af.rows         = b->pend_splits + 1;
-                af.row0         = b->pend_splits;
-                af.sum0         = b->pend_splits - 1;       /* the pending MAC folded its rows into this one */
-                af.flags       |= STEP_HEAD_ONLY;
-                /* A synchronous host call on the own stream: every launch that delivered an earlier
-                 * block has completed (the caller has its output), and the predecessor in the
-                 * stream is this batch's pending MAC, which never touches the caller's input block
-                 * -- the block is fetched and transformed under that MAC whatever the launch size. */
-                if ((st == b->stream) && (b->opt_pdl != 0) && (b->opt_early_src != 0))
-                    af.flags       |= STEP_EARLY_SRC;
-                CU(launch_mac(b, af, fp, nact, st, true, serial));
-            }
-            else
-                CU(launch_mac(b, a, plan, nact, st, true, serial));
-            b->pend_ready   = false;
-            b->last_was_frame = (st == b->stream) && (!b->profiling);
-            b->stats.launches       += 1;
-            b->stats.mac_stream_bytes += launch_bytes;
-        }
-        else
-        {
-            MacPlan sp      = plan;
-            sp.sh.bias      = 0;
-            b->pend_ready   = false;
-            b->la_live      = false;
-            b->stats.mac_stream_bytes += per_frame_bytes;
-            const bool ahead = (b->rank >= 14) && (b->opt_pdl != 0) && (!b->profiling) && (b->opt_chain_ahead != 0) && (frames == 1);
-            if (ahead)
-            {
-                /* Block-by-block callers at ranks 14..16: partitions q >= 1 of block t need complete frames
-                 * only, so their MAC is launched one block AHEAD -- behind the inverse transform of block
-                 * t - 1 -- into a row slot of its own, and streams under that inverse transform and under
-                 * the transform of block t; partition 0 is added by the inverse transform of block t
-                 * (STEP_Q0_IN_INV).  Stream order per call:  k_fwd(t)  k_inv(t)  k_mac(t + 1).
-                 * What orders them: chain_head ("frames < x are final", published by k_inv(t) once
-                 * k_fwd(t) has completed; k_mac(t + 1) polls it), row slots t mod FRAME_SLOTS, and one
-                 * CTA of every kernel that waits for the launch before it as its last instruction. */
-                const uint64_t t    = a.t_base + a.frame0;
-                const uint32_t t32  = uint32_t(t);
-                uint32_t *head      = b->d_ring_head + b->n;
-                auto mac_ahead = [&](uint64_t t_of, bool pdl) -> cudaError_t
-                {
-                    StepArgs am     = a;
-                    am.t_base       = t_of - a.frame0;
-                    am.ypart        = ypart_slot(b, uint32_t(t_of));
-                    am.flags       |= STEP_FROM_Q1 | STEP_AHEAD;
-                    am.chain_head   = head;
-                    return launch_mac(b, am, sp, nact, st, false, false, pdl);
-                };
-                if (!(b->ahead_valid && (b->ahead_t == t) && (b->ahead_splits == sp.splits)))
-                {
-                    /* cold start (or a MAC launched ahead for a block that never came): seed the chain head by
-                     * a copy and launch this block's MAC without the attribute -- both full dependencies */
-                    CU(cudaMemcpyAsync(head, &t32, sizeof(t32), cudaMemcpyHostToDevice, st));
-                    CU(mac_ahead(t, false));
-                    b->stats.launches += 1;
-                }
-                bool early = false, serial = false, dst_clash = false;
-                {
-                    const bool capable = (b->opt_early_src == 2) || ((b->opt_early_src == 1) && (st == b->stream));
-                    const BlockRows in  = { reinterpret_cast<uintptr_t>(src + f * F), stride * sizeof(float), F * sizeof(float), b->n };
-                    const BlockRows out = { reinterpret_cast<uintptr_t>(dst + f * F), dst_stride * sizeof(float), F * sizeof(float), b->n };
-                    hist_launch(st, b->device, capable, in, out, &early, &serial, &dst_clash);
-                }
-                StepArgs ai     = a;
-                ai.ypart        = ypart_slot(b, t32);
-                TRY(attach_park(b, ai, nact, st));      /* (may synchronise) */
-                StepArgs af     = a;
-                if (early)
-                    af.flags       |= STEP_EARLY_SRC;
-                CU(launch_fwd(af, nact, st, !serial));
-                ai.flags       |= STEP_Q0_IN_INV;
-                ai.chain_head   = head;
-                CU(launch_inv(ai, nact, st, true, b->d_tickets));
-                CU(mac_ahead(t + 1, true));
-                b->ahead_valid  = true;
-                b->ahead_t      = t + 1;
-                b->ahead_splits = sp.splits;
-                b->chain_valid  = true;
-                b->chain_next   = t32 + 1u;
-                b->stats.launches       += 3;
-                b->stats.mac_launches   += 1;
-                b->stats.mac_algo_bytes += per_frame_bytes;
-                b->stats.frames         += nact;
-                f              += 1;
-                continue;
-            }
-            b->ahead_valid  = false;
-            hist_reset(st, b->device);
-            /* Ranks 14..16: the three kernels of a block are chained with programmatic serialisation --
-             * the partition stream of q >= 1 runs beside the block's own transform (which only the
-             * stage with q = 0 needs, taken last, STEP_AFTER_FWD), table staging overlaps the launch
-             * before; every kernel orders itself with griddepcontrol.wait. */
-            const bool chain = (b->rank >= 14) && (b->opt_pdl != 0) && (!b->profiling);
-            TRY(attach_park(b, a, nact, st));       /* (may synchronise: before the chain starts) */
-            CU(launch_fwd(a, nact, st, chain));
-            StepArgs am     = a;
-            if (chain)
-                am.flags       |= STEP_AFTER_FWD;
-            {
-                /* "the spectra of all frames < t are final": published by the k_mac of block t - 1; whenever
-                 * that was not the launch before this one (first block, a multi-frame pass, the general
-                 * path, another frame counter) the word is seeded by a copy -- a full dependency */
-                const uint32_t t32 = uint32_t(a.t_base + a.frame0);
-                if ((!b->chain_valid) || (b->chain_next != t32))
-                    CU(cudaMemcpyAsync(b->d_ring_head + b->n, &t32, sizeof(t32), cudaMemcpyHostToDevice, st));
-                am.chain_head   = b->d_ring_head + b->n;
-                b->chain_valid  = true;
-                b->chain_next   = t32 + 1u;
-            }
-            CU(launch_mac(b, am, sp, nact, st, false, false, chain));
-            CU(launch_inv(a, nact, st, chain, b->d_tickets));      /* nact <= instances counters */
-            hist_unknown(st, b->device);
-            b->stats.launches       += 3;
-        }
-        b->stats.mac_launches   += 1;
-        b->stats.mac_algo_bytes += per_frame_bytes;
-        b->stats.frames         += nact;
-        f              += 1;
+        for (uint32_t k = (b->reduce.mode != 0) ? 0u : uint32_t(b->opt_multi); k >= 2; k >>= 1)
+            if (frames - f >= k) { tf = k; break; }
+        const int used  = (tf >= 2) ? step_multi(b, c, tf) : (fused && (!used_multi)) ? step_frame(b, c, f)
+                                                                                      : step_three(b, c, f);
+        if (used < 0)
+            return used;
+        used_multi     |= (tf >= 2);
+        f              += size_t(used);
     }
     if (used_multi)
         b->desc_dirty   = true;     /* ring_head was bypassed: re-seed before the next k_frame */
@@ -1956,9 +1978,9 @@ static int launch_pending_mac(Batch *b, cudaStream_t st)
     if (size_t(nact) * (plan.splits + 1) * F * sizeof(float2) > b->ypart_slot_bytes)
         return B200CONV_OK;                 /* sized by the next process call */
 
-    StepArgs a      = base_args(b);
+    Schedules &s    = b->sched;
+    StepArgs a      = base_args(b, 0);
     a.ypart         = ypart_slot(b, b->frame_seq);      /* the slot of the k_frame launch that will add partition 0 */
-    b->pend_seq     = b->frame_seq;
     a.splits        = plan.splits;
     a.rows          = plan.splits + 1;
     a.row0          = 0;
@@ -1973,17 +1995,15 @@ static int launch_pending_mac(Batch *b, cudaStream_t st)
     /* auto: early only while the caller keeps the GPU busy (the previous pending MAC was still
      * running when this call arrived); a caller that comes back once per audio block gets the
      * delivering launch to itself */
-    const bool early = (b->opt_pdl != 0) && b->last_was_frame &&
+    const bool early = (b->opt_pdl != 0) && s.pend.last_was_frame &&
                        ((b->opt_early_pend == 2) || ((b->opt_early_pend == 1) && b->caller_busy));
     if (early)
         a.flags        |= STEP_WAIT_HEAD;
     CU(launch_mac_raw(a, plan, nact, st, early));
-    b->last_was_frame = false;
+    sched_continue(b, SCHED_PEND);
+    s.pend          = { true, b->t_batch, plan.splits, b->frame_seq, false };
     b->stats.launches       += 1;
     b->stats.mac_launches   += 1;
-    b->pend_ready   = true;
-    b->pend_t       = b->t_batch;
-    b->pend_splits  = plan.splits;
     return B200CONV_OK;
 }
 
@@ -2023,12 +2043,12 @@ static int publish_jobs(Batch *b, const Job *list, size_t count, cudaStream_t st
  * A 256-sample call of a phase-shifted instance (BASELINE config 2) is P1 + FFT + MAC + P2 in one
  * k_frame<GEN> launch; a call inside a frame is one k_partial_fused launch. */
 static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const float *src, size_t stride,
-                                 size_t count, cudaStream_t st)
+                                 size_t count, cudaStream_t st, uint32_t mode)
 {
     const size_t F      = size_t(1) << (b->rank - 1);
     TRY(upload_tables(b, st));
     hist_reset(st, b->device);          /* every CTA of the job-list form waits for all earlier launches */
-    b->la_live          = false;        /* a lookahead schedule restarts with a priming group */
+    sched_continue(b, SCHED_NONE);
     std::vector<size_t> &pos = b->g_pos;
     std::vector<Job> &jobs = b->g_jobs;
     for (uint32_t i : b->active)
@@ -2151,7 +2171,7 @@ static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const 
         if (jobs.empty())
             break;
 
-        StepArgs a  = base_args(b);
+        StepArgs a  = base_args(b, mode);
         JobPack pack;
         TRY(publish_jobs(b, jobs.data(), jobs.size(), st, &pack, &a.jobs));
         a.n_jobs    = uint32_t(jobs.size());
@@ -2181,10 +2201,7 @@ static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const 
     }
 
     hist_unknown(st, b->device);
-    b->chain_valid = false;
-    b->ahead_valid = false;
     b->uniform_stale = true;    /* per-instance frame counters moved independently of t_batch */
-    b->pend_ready = false;
     return B200CONV_OK;
 }
 
@@ -2196,11 +2213,12 @@ static int process_general_fused(Batch *b, float *dst, size_t dst_stride, const 
  *                          frames about to start: partitions q >= 1 -> their pending block)
  * and each instance contributes at most one item per stage. */
 static int process_general_staged(Batch *b, float *dst, size_t dst_stride, const float *src, size_t stride,
-                                  size_t count, cudaStream_t st)
+                                  size_t count, cudaStream_t st, uint32_t mode)
 {
     const size_t F      = size_t(1) << (b->rank - 1);
     TRY(upload_tables(b, st));
     hist_reset(st, b->device);
+    sched_continue(b, SCHED_NONE);
     std::vector<size_t> &pos = b->g_pos;
     std::vector<Job> &fft = b->g_fft, &mac = b->g_mac, &part = b->g_part;
     for (uint32_t i : b->active)
@@ -2318,7 +2336,7 @@ static int process_general_staged(Batch *b, float *dst, size_t dst_stride, const
         }
         const Job *dj = b->d_jobs + at;
 
-        StepArgs a  = base_args(b);
+        StepArgs a  = base_args(b, mode);
         if (!part.empty())
         {
             a.jobs      = part_packed ? nullptr : dj;
@@ -2385,7 +2403,7 @@ static int process_general_staged(Batch *b, float *dst, size_t dst_stride, const
             a.jobs      = dj + part_up + fft.size();
             a.n_jobs    = uint32_t(mac.size());
             a.splits    = plan.splits;
-            CU(launch_mac(b, a, plan, a.n_jobs, st));
+            CU(launch_kmac(b, a, plan, a.n_jobs, st, false));
             TRY(attach_park(b, a, a.n_jobs, st));
             CU(launch_inv(a, a.n_jobs, st));
             b->stats.launches       += 2;
@@ -2398,23 +2416,16 @@ static int process_general_staged(Batch *b, float *dst, size_t dst_stride, const
     /* ring_head was bypassed and the per-instance frame counters moved: both matter only to a
      * k_frame launch, which refreshes the tables first (uniform_stale) */
     hist_unknown(st, b->device);
-    b->chain_valid = false;
-    b->ahead_valid = false;
     b->uniform_stale = true;
-    b->pend_ready = false;
     return B200CONV_OK;
 }
 
-static int process_general(Batch *b, float *dst, size_t dst_stride, const float *src, size_t stride,
-                           size_t count, cudaStream_t st)
-{
-    if ((b->opt_fused != 0) && (b->rank <= 13))
-        return process_general_fused(b, dst, dst_stride, src, stride, count, st);
-    return process_general_staged(b, dst, dst_stride, src, stride, count, st);
-}
-
-static int process_device2_impl(b200conv_batch_t *b, float *dst, size_t dst_stride,
-                                        const float *src, size_t src_stride, size_t count, void *stream)
+/* One process call on device-addressable matrices, on stream `st` (NULL: the batch's own stream);
+ * `mode`: CALL_*.  Out of host memory is B200CONV_ERR_NOMEM for every caller, the synchronous entry
+ * points included. */
+static int process_rows(b200conv_batch_t *b, float *dst, size_t dst_stride, const float *src, size_t src_stride,
+                        size_t count, cudaStream_t st, uint32_t mode)
+try
 {
     if (b == nullptr)
         return fail(B200CONV_ERR_ARG, "b200conv_process_device: NULL handle");
@@ -2423,10 +2434,10 @@ static int process_device2_impl(b200conv_batch_t *b, float *dst, size_t dst_stri
     if ((dst == nullptr) || (src == nullptr) || ((b->n > 1) && ((src_stride < count) || (dst_stride < count))))
         return fail(B200CONV_ERR_ARG, "b200conv_process_device: bad buffers");
     ENTER_DEVICE(b);
-    cudaStream_t st = (stream != nullptr) ? cudaStream_t(stream) : b->stream;
+    if (st == nullptr)
+        st = b->stream;
     TRY(check_device_error(b));
-    b->last_was_frame = false;
-    if (b->eager_call)
+    if (mode & CALL_SYNC)
     {
         b->caller_busy  = b->pend_inflight && (cudaEventQuery(b->ev_pend) == cudaErrorNotReady);
         cudaGetLastError();         /* "not ready" is an answer, not an error: do not leave it behind
@@ -2461,17 +2472,26 @@ static int process_device2_impl(b200conv_batch_t *b, float *dst, size_t dst_stri
 
     int rc;
     if (uniform)
-        rc = process_uniform(b, dst, dst_stride, src, src_stride, count / F, st);
+        rc = process_uniform(b, dst, dst_stride, src, src_stride, count / F, st, mode);
     else if (b->reduce.mode != 0)
         return fail(B200CONV_ERR_STATE, "the fused cross-GPU reduce handles whole-frame calls only");
+    else if ((b->opt_fused != 0) && (b->rank <= 13))
+        rc = process_general_fused(b, dst, dst_stride, src, src_stride, count, st, mode);
     else
-        rc = process_general(b, dst, dst_stride, src, src_stride, count, st);
+        rc = process_general_staged(b, dst, dst_stride, src, src_stride, count, st, mode);
     if ((rc == B200CONV_OK) && (st != b->stream))
     {
         CU(cudaEventRecord(b->ev_last, st));
         b->last_foreign = true;
     }
     return rc;
+}
+catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
+
+extern "C" int b200conv_process_device2(b200conv_batch_t *b, float *dst, size_t dst_stride,
+                                        const float *src, size_t src_stride, size_t count, void *stream)
+{
+    return process_rows(b, dst, dst_stride, src, src_stride, count, cudaStream_t(stream), 0);
 }
 
 extern "C" int b200conv_process_device(b200conv_batch_t *b, float *dst, const float *src,
@@ -2486,7 +2506,7 @@ static int finish_sync_call(Batch *b)
 {
     CU(cudaEventRecord(b->ev_done, b->stream));
     TRY(launch_pending_mac(b, b->stream));
-    if (b->pend_ready)
+    if (b->sched.pend.ready)
     {
         CU(cudaEventRecord(b->ev_pend, b->stream));
         b->pend_inflight = true;
@@ -2517,6 +2537,16 @@ static int ensure_staging(Batch *b, size_t floats)
     return B200CONV_OK;
 }
 
+/* samples per instance per pass of a staged synchronous call: bounded staging, at least one frame */
+static size_t sync_chunk(const Batch *b)
+{
+    size_t cap = (size_t(1) << 24) / b->n;
+    if (cap > 65536)    cap = 65536;
+    size_t F   = (b->rank > 0) ? (size_t(1) << (b->rank - 1)) : 128;
+    if (cap < F)        cap = F;
+    return (cap / F) * F;
+}
+
 extern "C" int b200conv_process(b200conv_batch_t *b, float *const *dst, const float *const *src,
                                 size_t count)
 {
@@ -2531,13 +2561,7 @@ extern "C" int b200conv_process(b200conv_batch_t *b, float *const *dst, const fl
             return fail(B200CONV_ERR_ARG, "b200conv_process: NULL buffer for instance %zu", i);
     ENTER_DEVICE(b);
 
-    /* samples per instance per pass: bounded staging, at least one frame */
-    size_t cap = (size_t(1) << 24) / b->n;
-    if (cap > 65536)    cap = 65536;
-    size_t F   = (b->rank > 0) ? (size_t(1) << (b->rank - 1)) : 128;
-    if (cap < F)        cap = F;
-    cap        = (cap / F) * F;
-
+    const size_t cap = sync_chunk(b);
     for (size_t done = 0; done < count; )
     {
         size_t c = count - done;
@@ -2550,22 +2574,14 @@ extern "C" int b200conv_process(b200conv_batch_t *b, float *const *dst, const fl
         /* the gathered block sits in page-locked memory: short blocks are read and written by the
          * kernels in place across PCIe (no copy operations in the stream), long ones are copied */
         const bool in_place = (b->opt_zero_copy != 0) && (b->n * c * sizeof(float) <= (size_t(4) << 20));
-        b->eager_call = true;
-        int rc;
         if (in_place)
-        {
-            b->host_io      = true;
-            rc              = b200conv_process_device(b, b->h_out_dev, b->h_in_dev, c, c, b->stream);
-            b->host_io      = false;
-        }
+            TRY(process_rows(b, b->h_out_dev, c, b->h_in_dev, c, c, b->stream, CALL_SYNC | CALL_HOST_IO));
         else
         {
             hist_reset(b->stream, b->device);
             CU(cudaMemcpyAsync(b->d_in, b->h_in, b->n * c * sizeof(float), cudaMemcpyHostToDevice, b->stream));
-            rc              = b200conv_process_device(b, b->d_out, b->d_in, c, c, b->stream);
+            TRY(process_rows(b, b->d_out, c, b->d_in, c, c, b->stream, CALL_SYNC));
         }
-        b->eager_call = false;
-        TRY(rc);
         if (!in_place)
             CU(cudaMemcpyAsync(b->h_out, b->d_out, b->n * c * sizeof(float), cudaMemcpyDeviceToHost, b->stream));
         if (done + c >= count)
@@ -2603,13 +2619,8 @@ extern "C" int b200conv_process_planar(b200conv_batch_t *b, float *dst, const fl
             (as.type == cudaMemoryTypeHost) && (ad.type == cudaMemoryTypeHost) &&
             (as.devicePointer != nullptr) && (ad.devicePointer != nullptr))
         {
-            b->eager_call = true;
-            b->host_io    = true;
-            int rc = b200conv_process_device(b, static_cast<float *>(ad.devicePointer),
-                                             static_cast<const float *>(as.devicePointer), stride, count, b->stream);
-            b->eager_call = false;
-            b->host_io    = false;
-            TRY(rc);
+            TRY(process_rows(b, static_cast<float *>(ad.devicePointer), stride, static_cast<const float *>(as.devicePointer),
+                             stride, count, b->stream, CALL_SYNC | CALL_HOST_IO));
             TRY(finish_sync_call(b));
             b->stats.h2d_bytes += b->n * count * sizeof(float);
             b->stats.d2h_bytes += b->n * count * sizeof(float);
@@ -2618,12 +2629,7 @@ extern "C" int b200conv_process_planar(b200conv_batch_t *b, float *dst, const fl
         cudaGetLastError();     /* pageable memory: not an error, take the staged path */
     }
 
-    size_t cap = (size_t(1) << 24) / b->n;
-    if (cap > 65536)    cap = 65536;
-    size_t F   = (b->rank > 0) ? (size_t(1) << (b->rank - 1)) : 128;
-    if (cap < F)        cap = F;
-    cap        = (cap / F) * F;
-
+    const size_t cap = sync_chunk(b);
     for (size_t done = 0; done < count; )
     {
         size_t c = count - done;
@@ -2633,10 +2639,7 @@ extern "C" int b200conv_process_planar(b200conv_batch_t *b, float *dst, const fl
         hist_reset(b->stream, b->device);
         CU(cudaMemcpy2DAsync(b->d_in, c * sizeof(float), src + done, stride * sizeof(float),
                              c * sizeof(float), b->n, cudaMemcpyHostToDevice, b->stream));
-        b->eager_call = true;
-        int rc = b200conv_process_device(b, b->d_out, b->d_in, c, c, b->stream);
-        b->eager_call = false;
-        TRY(rc);
+        TRY(process_rows(b, b->d_out, c, b->d_in, c, c, b->stream, CALL_SYNC));
         CU(cudaMemcpy2DAsync(dst + done, stride * sizeof(float), b->d_out, c * sizeof(float),
                              c * sizeof(float), b->n, cudaMemcpyDeviceToHost, b->stream));
         if (done + c >= count)
@@ -2783,7 +2786,7 @@ extern "C" int b200conv_set_profiling(b200conv_batch_t *b, int enable)
         return fail(B200CONV_ERR_ARG, "b200conv_set_profiling: NULL handle");
     b->profiling    = (enable != 0);
     b->desc_dirty   = true;     /* profiled launches are not pipelined: the slot counters are re-seeded */
-    b->pend_ready   = false;
+    sched_continue(b, SCHED_NONE);
     return B200CONV_OK;
 }
 
@@ -2816,7 +2819,7 @@ extern "C" int b200conv_set_option(b200conv_batch_t *b, const char *name, int va
     if ((b == nullptr) || (name == nullptr))
         return fail(B200CONV_ERR_ARG, "b200conv_set_option: bad arguments");
     if (!strcmp(name, "mac_splits") && (value >= 0) && (value <= 32))       b->tune_splits = value;
-    else if (!strcmp(name, "chain_ahead") && (value >= 0) && (value <= 1)) { b->opt_chain_ahead = value; b->ahead_valid = false; }
+    else if (!strcmp(name, "chain_ahead") && (value >= 0) && (value <= 1)) b->opt_chain_ahead = value;
     else if (!strcmp(name, "mac_tile") && ((value == 0) || (value == 256) || (value == 512) || (value == 1024))) g_tune_tile = value;
     else if (!strcmp(name, "mac_stages") && ((value == 0) || ((value >= 2) && (value <= 12)))) b->tune_stages = value;
     else if (!strcmp(name, "fused") && (value >= 0) && (value <= 1))        b->opt_fused = value;
@@ -2833,7 +2836,7 @@ extern "C" int b200conv_set_option(b200conv_batch_t *b, const char *name, int va
     else
         return fail(B200CONV_ERR_ARG, "b200conv_set_option: unknown option or bad value: %s = %d", name, value);
     b->desc_dirty   = true;     /* the hand-shake counters are re-seeded before the next launch */
-    b->pend_ready   = false;
+    sched_continue(b, SCHED_NONE);
     return B200CONV_OK;
 }
 
@@ -3364,13 +3367,6 @@ extern "C" int b200conv_init_many(b200conv_batch_t *b, size_t count, const size_
                                   const size_t *counts, size_t rank, const float *phases, const size_t *part_offsets)
 {
     try { return init_many_impl(b, count, idx, data, counts, rank, phases, part_offsets); }
-    catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
-}
-
-extern "C" int b200conv_process_device2(b200conv_batch_t *b, float *dst, size_t dst_stride,
-                                        const float *src, size_t src_stride, size_t count, void *stream)
-{
-    try { return process_device2_impl(b, dst, dst_stride, src, src_stride, count, stream); }
     catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
 }
 
