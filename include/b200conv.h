@@ -133,6 +133,42 @@ int     b200conv_init_shared(b200conv_batch_t *h, size_t idx, size_t src_idx, fl
 /* Convolver::destroy for instance `idx` (Convolver.cpp:71-75); idempotent. */
 int     b200conv_destroy(b200conv_batch_t *h, size_t idx);
 
+/* ---- impulse-response swap with crossfade ------------------------------------------------
+ *
+ *   b200conv_set_irs            replaces the IRs of running instances and KEEPS their input history:
+ *                               instance idx[k] gets data[k][0 .. counts[k]) (HOST pointers, borrowed
+ *                               for the call only).  With k counting samples of that instance from
+ *                               the first sample of its next process call and w(k) = min(1, (k + 1) /
+ *                               fade) (w = 1 when fade == 0: a hard switch), the instance outputs
+ *                               (1 - w) * (h_old (*) x) + w * (h_new (*) x), both convolutions over
+ *                               the whole input history since init.  Any process entry point, call
+ *                               size and phase; a fade may end inside a call.  Once w reaches 1 the
+ *                               new IR stays: get_state / get_dump report its conv_size, bins and
+ *                               partitions, while frames, frame_off and the phase go on unchanged.
+ *                               B200CONV_ERR_ARG: index out of range or twice, NULL data, counts[k]
+ *                               == 0 (a one-tap zero IR fades an instance out), or an IR of more
+ *                               partitions than the instance's ring reaches (ceil(count / F) + 1 >
+ *                               its partitions: use init).  B200CONV_ERR_STATE: an instance is not
+ *                               initialised, is already fading or lends its IR spectra
+ *                               (b200conv_init_shared), or the batch is reduce-connected.  A borrower
+ *                               may fade; afterwards it owns its spectra.  On any error nothing
+ *                               changes; count == 0 is a no-op.  Synchronous like b200conv_init: it
+ *                               waits for the work enqueued on the batch and for the new IRs' ingest.
+ *                               init / init_many / init_shared / destroy of a fading instance end its
+ *                               fade.  While instances fade, every process call also runs their new
+ *                               IRs through an internal second batch and blends (DESIGN.md §4.8); the
+ *                               synchronous entry points stage through device buffers.  The process
+ *                               call in which a fade ends (any entry point, process_device included)
+ *                               waits on the host for everything the batch has enqueued before it
+ *                               returns: the old IR's buffers are released there.
+ *                               b200conv_reduce_prepare / _connect refuse a fading batch
+ *                               (B200CONV_ERR_STATE).
+ *   b200conv_fade_remaining     samples of instance idx's fade not yet covered by the calls made so
+ *                               far (0: not fading); host arithmetic, never waits */
+int     b200conv_set_irs(b200conv_batch_t *h, size_t count, const size_t *idx, const float *const *data,
+                         const size_t *counts, size_t fade);
+size_t  b200conv_fade_remaining(const b200conv_batch_t *h, size_t idx);
+
 /* ---- Convolver::process ---------------------------------------------------------------- */
 
 /* N x Convolver::process(dst[i], src[i], count) (Convolver.cpp:217-313) in one call: HOST

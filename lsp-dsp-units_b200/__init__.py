@@ -60,7 +60,7 @@ def build(verbose=False):
     src = os.path.join(_HERE, "csrc", "engine.cu")
     deps = [src, os.path.join(_ROOT, "include", "b200conv.h")] + [
         os.path.join(_HERE, "csrc", h) for h in ("kernels.cuh", "equalizer.cuh", "spectral.cuh", "spectral_host.cuh",
-                                                  "splitter.cuh", "matrix.cuh", "matrix_host.cuh")]
+                                                  "splitter.cuh", "matrix.cuh", "matrix_host.cuh", "batch_fade.cuh")]
     if os.path.exists(LIB_PATH) and all(os.path.getmtime(LIB_PATH) >= os.path.getmtime(d) for d in deps):
         return LIB_PATH
     cmd = ["nvcc"] + NVCC_FLAGS + ["-I", os.path.join(_ROOT, "include"), "-o", LIB_PATH, src]
@@ -83,6 +83,8 @@ _SIGNATURES = {
                                           _FP, ctypes.POINTER(_SZ)]),
     "b200conv_init_shared": (ctypes.c_int, [_VP, _SZ, _SZ, ctypes.c_float]),
     "b200conv_destroy": (ctypes.c_int, [_VP, _SZ]),
+    "b200conv_set_irs": (ctypes.c_int, [_VP, _SZ, ctypes.POINTER(_SZ), ctypes.POINTER(_FP), ctypes.POINTER(_SZ), _SZ]),
+    "b200conv_fade_remaining": (_SZ, [_VP, _SZ]),
     "b200conv_process": (ctypes.c_int, [_VP, ctypes.POINTER(_FP), ctypes.POINTER(_FP), _SZ]),
     "b200conv_process_planar": (ctypes.c_int, [_VP, _VP, _VP, _SZ, _SZ]),
     "b200conv_process_device": (ctypes.c_int, [_VP, _VP, _VP, _SZ, _SZ, _VP]),
@@ -252,6 +254,21 @@ class ConvolverBatch:
 
     def destroy(self, idx):
         _check(lib().b200conv_destroy(self._h, idx))
+
+    # -- impulse-response swap with crossfade ---------------------------------------------------
+    def set_irs(self, indices, irs, fade=0):
+        """New impulse responses for running instances, keeping their input history: over the next
+        ``fade`` samples each output moves linearly from the old IR's to the new one's
+        (``b200conv_set_irs``; synchronous, like ``init``)."""
+        irs = [np.ascontiguousarray(x, dtype=np.float32) for x in irs]
+        n = len(indices)
+        assert len(irs) == n
+        _check(lib().b200conv_set_irs(self._h, n, (_SZ * n)(*indices), (_FP * n)(*[_ptr(x) for x in irs]),
+                                      (_SZ * n)(*[x.size for x in irs]), fade))
+
+    def fade_remaining(self, idx):
+        """Samples of instance ``idx``'s fade not yet covered by the calls made so far (0: not fading)."""
+        return int(lib().b200conv_fade_remaining(self._h, idx))
 
     # -- Convolver::process -------------------------------------------------------------------
     def process(self, src, out=None):

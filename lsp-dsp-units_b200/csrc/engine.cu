@@ -10,6 +10,7 @@
  */
 #include "b200conv.h"
 #include "kernels.cuh"
+#include "batch_fade.cuh"
 
 #include <chrono>
 #include <cmath>
@@ -602,6 +603,8 @@ struct Slab                         /* one device allocation shared by the insta
     size_t      refs        = 0;
 };
 static void slab_release(Slab *s);
+struct b200conv_batch;
+static int fade_discard(b200conv_batch *b, size_t idx);
 
 struct Instance
 {
@@ -748,6 +751,14 @@ struct b200conv_batch
     bool                    profiling   = false;
     std::vector<cudaEvent_t> prof_events;           /* pairs: before / after each k_mac */
     size_t                  prof_used   = 0;
+
+    /* crossfade to new impulse responses (b200conv_set_irs, DESIGN.md §4.8) */
+    b200conv_batch         *twin        = nullptr;  /* the fading instances with their new IRs, one slot each */
+    std::vector<FadeRow>    fades;                  /* by twin slot */
+    FadeRow                *d_fades     = nullptr;  /* device copy of `fades` (set_irs sizes it) */
+    float                  *fade_in     = nullptr, *fade_out = nullptr;    /* [slot][count] */
+    size_t                  fade_floats = 0;
+    uint64_t                fade_clock  = 0;        /* samples per instance processed while fades ran */
 };
 
 typedef b200conv_batch Batch;
@@ -1190,6 +1201,10 @@ extern "C" void b200conv_free(b200conv_batch_t *b)
         return;
     DeviceScope device_scope_(b->device);
     quiesce(b);
+    b200conv_free(b->twin);
+    if (b->d_fades)     cudaFree(b->d_fades);
+    if (b->fade_in)     cudaFree(b->fade_in);
+    if (b->fade_out)    cudaFree(b->fade_out);
     for (Instance &in : b->inst)
         free_instance_buffers(in);
     for (float2 *t : b->tw)
@@ -1228,6 +1243,60 @@ extern "C" void b200conv_free(b200conv_batch_t *b)
 }
 
 /* ------------------------------------------------------------------------------------------- */
+/* crossfade bookkeeping (b200conv_set_irs)                                                     */
+
+static bool fading(const Batch *b)
+{
+    return b->twin != nullptr;
+}
+
+/* the twin slot of instance idx, or -1 when it is not fading */
+static long fade_slot(const Batch *b, size_t idx)
+{
+    for (size_t s = 0; s < b->fades.size(); ++s)
+        if (b->fades[s].row == int64_t(idx))
+            return long(s);
+    return -1;
+}
+
+/* After fades ended (the batch and its twin are quiesced): frees the twin and the fade buffers when
+ * no fade is left, else refreshes the twin's tables and the device copy of `fades` (same size). */
+static int fade_tables(Batch *b)
+{
+    bool live = false;
+    for (const FadeRow &r : b->fades)
+        live   |= (r.row >= 0);
+    if (!live)
+    {
+        b200conv_free(b->twin);
+        if (b->d_fades)     cudaFree(b->d_fades);
+        if (b->fade_in)     cudaFree(b->fade_in);
+        if (b->fade_out)    cudaFree(b->fade_out);
+        b->twin         = nullptr;
+        b->fades.clear();
+        b->d_fades      = nullptr;
+        b->fade_in      = b->fade_out = nullptr;
+        b->fade_floats  = 0;
+        return B200CONV_OK;
+    }
+    rebuild_tables(b->twin);
+    CU(cudaMemcpyAsync(b->d_fades, b->fades.data(), b->fades.size() * sizeof(FadeRow), cudaMemcpyHostToDevice, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    return B200CONV_OK;
+}
+
+/* init / destroy of instance idx (the batch is quiesced): its fade, if any, ends without a handover */
+static int fade_discard(Batch *b, size_t idx)
+{
+    const long s    = fade_slot(b, idx);
+    if (s < 0)
+        return B200CONV_OK;
+    TRY(b200conv_destroy(b->twin, size_t(s)));
+    b->fades[size_t(s)].row = -1;
+    return fade_tables(b);
+}
+
+/* ------------------------------------------------------------------------------------------- */
 /* init / destroy                                                                               */
 
 extern "C" int b200conv_destroy(b200conv_batch_t *b, size_t idx)
@@ -1242,6 +1311,7 @@ extern "C" int b200conv_destroy(b200conv_batch_t *b, size_t idx)
                     idx, in.g_sharers);
     ENTER_DEVICE(b);
     CU(quiesce(b));
+    TRY(fade_discard(b, idx));
     if (in.g_owner >= 0)
         b->inst[size_t(in.g_owner)].g_sharers -= 1;
     free_instance_buffers(in);
@@ -1553,6 +1623,8 @@ static int init_many_impl(b200conv_batch_t *b, size_t count, const size_t *idx, 
         in              = (counts[k] == 0) ? Instance() : fresh[slot++];
     }
     rebuild_tables(b);
+    for (size_t k = 0; k < count; ++k)
+        TRY(fade_discard(b, idx[k]));
     return B200CONV_OK;
 }
 
@@ -1585,6 +1657,8 @@ static int init_shared_impl(b200conv_batch_t *b, size_t idx, size_t src_idx, flo
         return fail(B200CONV_ERR_STATE, "b200conv_init_shared: instance %zu is not initialised", src_idx);
     if (b->inst[idx].g_sharers > 0)
         return fail(B200CONV_ERR_STATE, "instance %zu lends its IR spectra to other instances: destroy those first", idx);
+    if (fade_slot(b, owner) >= 0)
+        return fail(B200CONV_ERR_STATE, "b200conv_init_shared: instance %zu is fading to a new impulse response", owner);
 
     ENTER_DEVICE(b);
     CU(quiesce(b));
@@ -1634,6 +1708,246 @@ static int init_shared_impl(b200conv_batch_t *b, size_t idx, size_t src_idx, flo
     in.frames       = 0;
     in.pend_valid   = false;
     rebuild_tables(b);
+    return fade_discard(b, idx);
+}
+
+/* ------------------------------------------------------------------------------------------- */
+/* crossfade to new impulse responses (b200conv_set_irs, DESIGN.md §4.8)                        */
+
+/* The output of a convolver depends on its impulse response only through G and the pending block
+ * (aux: pend); the ring and the frame in progress (aux: cur) hold the input alone.  So the twin
+ * instance at slot first + k, just initialised with the new IR, continues instance idx[k] exactly
+ * as if it had always had that IR once it holds the same ring rows, frame in progress and
+ * counters; its pending block is recomputed with the new G by the next call that needs it
+ * (pend_valid = false).  Both batches are quiesced. */
+static inline uint32_t slot_of(const Instance &in, uint64_t t);
+
+static int fade_clone(Batch *b, Batch *tw, const size_t *idx, size_t count, size_t first)
+{
+    cudaStream_t st = tw->stream;
+    for (size_t k = 0; k < count; ++k)
+    {
+        const Instance &from = b->inst[idx[k]];
+        Instance &to    = tw->inst[first + k];
+        const size_t F  = from.F;
+        /* the last min(frames, S_new) complete frames: frame t sits in slot (-t) mod S, so going back
+         * in time both slot indices rise by one and a run ends where either ring wraps */
+        const uint64_t m = std::min<uint64_t>(from.frames, to.S);
+        for (uint64_t j = 0; j < m; )
+        {
+            const uint64_t t    = from.frames - 1 - j;
+            const uint64_t s0   = slot_of(from, t), s1 = slot_of(to, t);
+            const uint64_t run  = std::min<uint64_t>(m - j, std::min<uint64_t>(from.S - s0, to.S - s1));
+            CU(cudaMemcpyAsync(to.ring + s1 * F, from.ring + s0 * F, run * F * sizeof(float2), cudaMemcpyDeviceToDevice, st));
+            j              += run;
+        }
+        CU(cudaMemcpyAsync(to.aux, from.aux, F * sizeof(float), cudaMemcpyDeviceToDevice, st));    /* cur */
+        to.off          = from.off;
+        to.off0         = from.off0;
+        to.frames       = from.frames;
+        to.pend_valid   = false;
+    }
+    CU(cudaStreamSynchronize(st));
+    return B200CONV_OK;
+}
+
+static bool fade_done(const Batch *b, const FadeRow &r)
+{
+    return (r.row >= 0) && ((r.fade <= 1) || (b->fade_clock - r.start >= r.fade));
+}
+
+/* Hands over every fade whose weight has reached 1: the instance becomes its twin instance (new G,
+ * ring, frame buffers and slab reference; the same counters), and its old buffers are released
+ * (a borrowed G stays with its owner).  Waits for everything enqueued first: the old buffers may
+ * still be read by launches in flight. */
+static int fade_handover(Batch *b)
+{
+    bool due = false;
+    for (const FadeRow &r : b->fades)
+        due    |= fade_done(b, r);
+    if (!due)
+        return B200CONV_OK;
+    CU(quiesce(b));
+    CU(quiesce(b->twin));
+    for (size_t s = 0; s < b->fades.size(); ++s)
+    {
+        FadeRow &r      = b->fades[s];
+        if (!fade_done(b, r))
+            continue;
+        Instance &in    = b->inst[size_t(r.row)];
+        if (in.g_owner >= 0)
+            b->inst[size_t(in.g_owner)].g_sharers -= 1;
+        free_instance_buffers(in);
+        in              = b->twin->inst[s];
+        b->twin->inst[s] = Instance();
+        r.row           = -1;
+    }
+    rebuild_tables(b);
+    return fade_tables(b);
+}
+
+static int set_irs_impl(b200conv_batch_t *b, size_t count, const size_t *idx, const float *const *data,
+                        const size_t *counts, size_t fade)
+{
+    if (b == nullptr)
+        return fail(B200CONV_ERR_ARG, "b200conv_set_irs: NULL handle");
+    if (count == 0)
+        return B200CONV_OK;
+    if ((idx == nullptr) || (data == nullptr) || (counts == nullptr))
+        return fail(B200CONV_ERR_ARG, "b200conv_set_irs: bad arguments");
+    std::vector<char> seen(b->n, 0);
+    for (size_t k = 0; k < count; ++k)
+    {
+        if ((idx[k] >= b->n) || seen[idx[k]])
+            return fail(B200CONV_ERR_ARG, "b200conv_set_irs: index %zu out of range or repeated", idx[k]);
+        seen[idx[k]]    = 1;
+        if ((data[k] == nullptr) || (counts[k] == 0))
+            return fail(B200CONV_ERR_ARG, "b200conv_set_irs: NULL or empty impulse response for instance %zu", idx[k]);
+    }
+    if (b->reduce.mode != 0)
+        return fail(B200CONV_ERR_STATE, "b200conv_set_irs: the batch is connected to a cross-GPU reduce");
+    for (size_t k = 0; k < count; ++k)
+    {
+        const Instance &in = b->inst[idx[k]];
+        if (!in.active)
+            return fail(B200CONV_ERR_STATE, "b200conv_set_irs: instance %zu is not initialised", idx[k]);
+        if (fade_slot(b, idx[k]) >= 0)
+            return fail(B200CONV_ERR_STATE, "b200conv_set_irs: instance %zu is already fading", idx[k]);
+        if (in.g_sharers > 0)
+            return fail(B200CONV_ERR_STATE, "b200conv_set_irs: instance %zu lends its IR spectra to %zu other instance(s)",
+                        idx[k], in.g_sharers);
+        if ((counts[k] + in.F - 1) / in.F + 1 > in.nq)
+            return fail(B200CONV_ERR_ARG, "b200conv_set_irs: %zu taps need more partitions than instance %zu's ring "
+                        "reaches (%zu): use b200conv_init", counts[k], idx[k], in.nq);
+    }
+
+    ENTER_DEVICE(b);
+    CU(quiesce(b));
+    if (fading(b))
+        CU(quiesce(b->twin));
+
+    /* a new twin: the fades still running keep their order, the new ones follow */
+    std::vector<size_t> keep;
+    for (size_t s = 0; s < b->fades.size(); ++s)
+        if (b->fades[s].row >= 0)
+            keep.push_back(s);
+    const size_t first = keep.size();
+    Batch *tw       = nullptr;
+    TRY(create_impl(&tw, b->device, first + count));
+    tw->tune_splits = b->tune_splits;       tw->tune_stages     = b->tune_stages;
+    tw->opt_fused   = b->opt_fused;         tw->opt_bias        = b->opt_bias;
+    tw->opt_pdl     = b->opt_pdl;           tw->opt_zero_copy   = b->opt_zero_copy;
+    tw->opt_multi   = b->opt_multi;         tw->opt_early_src   = b->opt_early_src;
+    tw->opt_chain_ahead = b->opt_chain_ahead;
+    tw->opt_lookahead = b->opt_lookahead;   tw->opt_eager       = b->opt_eager;
+    tw->opt_early_pend = b->opt_early_pend;
+    std::vector<size_t> slots(count), offsets(count);
+    for (size_t k = 0; k < count; ++k)
+    {
+        slots[k]        = first + k;
+        offsets[k]      = b->inst[idx[k]].q_lo;
+    }
+    std::vector<FadeRow> rows(first + count);
+    for (size_t j = 0; j < first; ++j)
+        rows[j]         = b->fades[keep[j]];
+    for (size_t k = 0; k < count; ++k)
+        rows[first + k] = { int64_t(idx[k]), b->fade_clock, uint64_t(fade) };
+
+    /* everything that can fail comes before the batch changes: the twin, the clone, the row table */
+    FadeRow *d_rows = nullptr;
+    int rc          = init_many_impl(tw, count, slots.data(), data, counts, b->rank, nullptr, offsets.data());
+    if (rc == B200CONV_OK)
+        rc              = fade_clone(b, tw, idx, count, first);
+    if (rc == B200CONV_OK)
+    {
+        cudaError_t e   = cudaMalloc(&d_rows, rows.size() * sizeof(FadeRow));
+        if (e == cudaSuccess)
+            e               = cudaMemcpy(d_rows, rows.data(), rows.size() * sizeof(FadeRow), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess)
+        {
+            cudaGetLastError();
+            rc              = fail((e == cudaErrorMemoryAllocation) ? B200CONV_ERR_NOMEM : B200CONV_ERR_CUDA,
+                                   "b200conv_set_irs: fade table: %s", cudaGetErrorString(e));
+        }
+    }
+    if (rc != B200CONV_OK)
+    {
+        std::string keep_error = g_last_error;
+        if (d_rows) cudaFree(d_rows);
+        b200conv_free(tw);
+        g_last_error    = keep_error;
+        return rc;
+    }
+
+    /* commit: the running fades' instances move into the new twin */
+    for (size_t j = 0; j < first; ++j)
+    {
+        tw->inst[j]     = b->twin->inst[keep[j]];
+        b->twin->inst[keep[j]] = Instance();
+    }
+    b200conv_free(b->twin);
+    if (b->d_fades) cudaFree(b->d_fades);
+    b->twin         = tw;
+    b->fades.swap(rows);
+    b->d_fades      = d_rows;
+    rebuild_tables(tw);
+    return fade_handover(b);                /* fade <= 1: the new IR at once */
+}
+
+extern "C" size_t b200conv_fade_remaining(const b200conv_batch_t *b, size_t idx)
+{
+    if ((b == nullptr) || (idx >= b->n))
+        return 0;
+    const long s    = fade_slot(b, idx);
+    if (s < 0)
+        return 0;
+    const FadeRow &r = b->fades[size_t(s)];
+    const uint64_t done = b->fade_clock - r.start;
+    return (done < r.fade) ? size_t(r.fade - done) : 0;
+}
+
+static int process_rows(b200conv_batch_t *b, float *dst, size_t dst_stride, const float *src, size_t src_stride,
+                        size_t count, cudaStream_t st, uint32_t mode);
+
+static dim3 fade_grid(size_t slots, size_t count)
+{
+    const size_t x  = (count + 255) / 256;
+    return dim3(uint32_t((x < 64) ? x : 64), uint32_t((slots < 65535) ? slots : 65535));
+}
+
+/* A call during a fade, before the batch's own launches (which may overwrite src): the fading rows
+ * of src -> fade_in, the twin's call on them -> fade_out.  The gather is a full dependency that
+ * does not trigger its successor early; the launch history of the stream learns nothing of it. */
+static int fade_before(Batch *b, const float *src, size_t src_stride, size_t count, cudaStream_t st)
+{
+    const size_t slots  = b->fades.size();
+    if (slots * count > b->fade_floats)
+    {
+        CU(quiesce(b));
+        CU(cudaStreamSynchronize(st));
+        if (b->fade_in)     cudaFree(b->fade_in);
+        if (b->fade_out)    cudaFree(b->fade_out);
+        b->fade_in      = b->fade_out = nullptr;
+        b->fade_floats  = 0;
+        CU(cudaMalloc(&b->fade_in, slots * count * sizeof(float)));
+        CU(cudaMalloc(&b->fade_out, slots * count * sizeof(float)));
+        b->fade_floats  = slots * count;
+    }
+    k_fade_gather<<<fade_grid(slots, count), 256, 0, st>>>(b->fade_in, src, src_stride, b->d_fades, uint32_t(slots), count);
+    CU(cudaGetLastError());
+    hist_unknown(st, b->device);
+    return process_rows(b->twin, b->fade_out, count, b->fade_in, count, count, st, 0);
+}
+
+/* ... and after them: the fading rows of dst move towards the twin's output */
+static int fade_after(Batch *b, float *dst, size_t dst_stride, size_t count, cudaStream_t st)
+{
+    const size_t slots  = b->fades.size();
+    k_fade_blend<<<fade_grid(slots, count), 256, 0, st>>>(dst, dst_stride, b->fade_out, b->d_fades, uint32_t(slots),
+                                                          count, b->fade_clock);
+    CU(cudaGetLastError());
+    hist_unknown(st, b->device);
+    b->fade_clock  += count;
     return B200CONV_OK;
 }
 
@@ -2445,6 +2759,9 @@ try
     }
     if (b->pend_inflight && (st != b->stream))
         CU(cudaStreamWaitEvent(st, b->ev_pend, 0));     /* a pending MAC may still be running on the own stream */
+    const bool fade = fading(b);
+    if (fade)
+        TRY(fade_before(b, src, src_stride, count, st));
 
     /* not initialised -> zeros (Convolver.cpp:219-223) */
     if (b->active.size() < b->n)
@@ -2479,11 +2796,15 @@ try
         rc = process_general_fused(b, dst, dst_stride, src, src_stride, count, st, mode);
     else
         rc = process_general_staged(b, dst, dst_stride, src, src_stride, count, st, mode);
+    if ((rc == B200CONV_OK) && fade)
+        rc = fade_after(b, dst, dst_stride, count, st);
     if ((rc == B200CONV_OK) && (st != b->stream))
     {
         CU(cudaEventRecord(b->ev_last, st));
         b->last_foreign = true;
     }
+    if ((rc == B200CONV_OK) && fade)
+        rc = fade_handover(b);
     return rc;
 }
 catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
@@ -2505,7 +2826,8 @@ extern "C" int b200conv_process_device(b200conv_batch_t *b, float *dst, const fl
 static int finish_sync_call(Batch *b)
 {
     CU(cudaEventRecord(b->ev_done, b->stream));
-    TRY(launch_pending_mac(b, b->stream));
+    if (!fading(b))                     /* during a fade the twin's launches come first in every call */
+        TRY(launch_pending_mac(b, b->stream));
     if (b->sched.pend.ready)
     {
         CU(cudaEventRecord(b->ev_pend, b->stream));
@@ -2573,7 +2895,7 @@ extern "C" int b200conv_process(b200conv_batch_t *b, float *const *dst, const fl
                 memcpy(b->h_in + i * c, src[i] + done, c * sizeof(float));
         /* the gathered block sits in page-locked memory: short blocks are read and written by the
          * kernels in place across PCIe (no copy operations in the stream), long ones are copied */
-        const bool in_place = (b->opt_zero_copy != 0) && (b->n * c * sizeof(float) <= (size_t(4) << 20));
+        const bool in_place = (b->opt_zero_copy != 0) && (b->n * c * sizeof(float) <= (size_t(4) << 20)) && (!fading(b));
         if (in_place)
             TRY(process_rows(b, b->h_out_dev, c, b->h_in_dev, c, c, b->stream, CALL_SYNC | CALL_HOST_IO));
         else
@@ -2612,7 +2934,7 @@ extern "C" int b200conv_process_planar(b200conv_batch_t *b, float *dst, const fl
      * read the input block and write the output block across PCIe themselves -- the input fetch
      * hides under the first partition stages, and two copy operations (and their launch
      * latencies) disappear from the call. */
-    if (b->opt_zero_copy)
+    if (b->opt_zero_copy && (!fading(b)))
     {
         cudaPointerAttributes as, ad;
         if ((cudaPointerGetAttributes(&as, src) == cudaSuccess) && (cudaPointerGetAttributes(&ad, dst) == cudaSuccess) &&
@@ -2837,6 +3159,8 @@ extern "C" int b200conv_set_option(b200conv_batch_t *b, const char *name, int va
         return fail(B200CONV_ERR_ARG, "b200conv_set_option: unknown option or bad value: %s = %d", name, value);
     b->desc_dirty   = true;     /* the hand-shake counters are re-seeded before the next launch */
     sched_continue(b, SCHED_NONE);
+    if (fading(b))
+        return b200conv_set_option(b->twin, name, value);
     return B200CONV_OK;
 }
 
@@ -2860,6 +3184,8 @@ extern "C" int b200conv_reduce_prepare(b200conv_batch_t *b, int grank, int world
         return fail(B200CONV_ERR_ARG, "b200conv_reduce_prepare: bad arguments");
     if ((b->rank == 0) || (b->rank > 13))
         return fail(B200CONV_ERR_STATE, "b200conv_reduce_prepare: initialise the instances first (ranks 8..13)");
+    if (fading(b))
+        return fail(B200CONV_ERR_STATE, "b200conv_reduce_prepare: instances are fading to new impulse responses");
     static_assert(sizeof(cudaIpcMemHandle_t) == B200CONV_IPC_HANDLE_BYTES, "IPC handle size");
     ENTER_DEVICE(b);
     TRY(b200conv_reduce_disconnect(b));
@@ -2892,6 +3218,8 @@ extern "C" int b200conv_reduce_connect(b200conv_batch_t *b, const unsigned char 
 {
     if ((b == nullptr) || (all_handles == nullptr) || (b->xchg == nullptr))
         return fail(B200CONV_ERR_ARG, "b200conv_reduce_connect: call b200conv_reduce_prepare first");
+    if (fading(b))
+        return fail(B200CONV_ERR_STATE, "b200conv_reduce_connect: instances are fading to new impulse responses");
     ENTER_DEVICE(b);
     CU(quiesce(b));
     ReduceArgs &r = b->reduce;
@@ -3367,6 +3695,13 @@ extern "C" int b200conv_init_many(b200conv_batch_t *b, size_t count, const size_
                                   const size_t *counts, size_t rank, const float *phases, const size_t *part_offsets)
 {
     try { return init_many_impl(b, count, idx, data, counts, rank, phases, part_offsets); }
+    catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
+}
+
+extern "C" int b200conv_set_irs(b200conv_batch_t *b, size_t count, const size_t *idx, const float *const *data,
+                                const size_t *counts, size_t fade)
+{
+    try { return set_irs_impl(b, count, idx, data, counts, fade); }
     catch (const std::bad_alloc &) { return fail(B200CONV_ERR_NOMEM, "out of host memory"); }
 }
 

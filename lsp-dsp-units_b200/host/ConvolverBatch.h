@@ -40,6 +40,13 @@ namespace b200conv
             /** Convolver::destroy for instance idx */
             void destroy(size_t idx)                { b200conv_destroy(pBatch, idx); }
 
+            /** New impulse responses for running instances idx[0 .. count), crossfaded over fade samples */
+            bool set_irs(size_t count, const size_t *idx, const float * const *data, const size_t *counts, size_t fade)
+                { return b200conv_set_irs(pBatch, count, idx, data, counts, fade) == B200CONV_OK; }
+
+            /** Samples of instance idx's crossfade still to come (0: not fading) */
+            size_t fade_remaining(size_t idx) const { return b200conv_fade_remaining(pBatch, idx); }
+
             /** N x Convolver::process with host buffers, synchronous */
             bool process(float * const *dst, const float * const *src, size_t count)
                 { return b200conv_process(pBatch, dst, src, count) == B200CONV_OK; }
