@@ -428,12 +428,47 @@ size_t  b200conv_eq_instances(const b200conv_eq_t *e);
  *                             spectrum[k] *= g[k] (`gain`: 2^rank real values, host).  Any table is
  *                             allowed -- the result is Re(IFFT(X H)) exactly as the reference's with
  *                             that callback.  Unbound (:174-175): the frames are only windowed.
+ *   b200conv_sp_set_function  the caller's own spectral function, run on the device between the
+ *   b200conv_sp_bind_function forward and inverse transforms (below).  ONE function per object;
+ *                             bind_function(idx) hands instance idx's frames to it (replacing a
+ *                             table), b200conv_sp_unbind unbinds.  bind_function without a function
+ *                             set, or set_function(NULL) while instances are bound, returns
+ *                             B200CONV_ERR_STATE; a non-NULL function may be replaced at any time.
+ *                             A function binding survives set_rank (pFunc does); tables do not.
  *   b200conv_sp_process_*     SpectralProcessor::process(dst, src, count) (:143-199) for all
  *                             instances: device matrices [instances][stride] (stream-ordered, dst ==
  *                             src allowed) or one planar host matrix (synchronous)
  *   b200conv_sp_reset         reset() (:247-257);  b200conv_sp_remaining  remaining() (:241-245);
- *   b200conv_sp_latency       latency() = 2^rank */
+ *   b200conv_sp_latency       latency() = 2^rank
+ *
+ * The spectral function.  For every frame of a function-bound instance, at the frame boundary where
+ * the reference calls pFunc: X = FFT_N(inb * w) (N = 2^rank, unscaled); the function edits X in
+ * place; then outb += Re(IFFT_N(X)) / N * w.  X may be left non-Hermitian: only Re(IFFT(X)) is
+ * used, as in the reference, i.e. the inverse of (X[k] + conj(X[N - k])) / 2.  The function is
+ * called ON THE CALLING THREAD inside b200conv_sp_process_device / _planar, after the forward
+ * transforms of its frames have been enqueued and before their inverse transforms are:
+ *     fn(user, spectra, frames_dev, frames_host, nframes, rank, stream)
+ *   spectra       DEVICE array [nframes][2^rank] of packed complex bins (re, im interleaved)
+ *   frames_dev    DEVICE copy of the frame table, frames_host the same table in host memory:
+ *   frames_host   frame f is spectra[f]; frames are ordered by instance, then time (every frame of
+ *                 the lowest bound instance first); `pos` is the sample index, counted from the
+ *                 first sample of the caller's process call, at which the reference calls pFunc
+ *   stream        the call's stream (the caller's for process_device, otherwise the object's).  The
+ *                 function enqueues its work there or orders it after that stream; the spectra are
+ *                 read when the stream reaches the inverse transforms.  All pointers are valid
+ *                 until the function returns.  A call into the same object from inside the
+ *                 function fails with B200CONV_ERR_STATE.
+ * Chunking: a call is cut into sub-calls of L = P * max(1, floor(2^25 / (B * N))) samples from its
+ * first sample (P = N / 2 the hop, B the number of function-bound instances); the function runs once
+ * per sub-call that holds frames, in time order.  Any P consecutive samples hold exactly one frame
+ * per instance, so one invocation carries at most max(2^25, B * N) bins (256 MiB unless one frame
+ * per bound instance needs more).  process_planar stages min(2^20, 2^24 / instances) samples at a
+ * time, rounded down to a multiple of L where L fits; where L does not, the staging boundaries
+ * cut sub-calls too.  A call with no function-bound instance calls nothing. */
 typedef struct b200conv_sp b200conv_sp_t;
+typedef struct b200conv_sp_frame { uint32_t instance; uint32_t pos; } b200conv_sp_frame_t;
+typedef void (*b200conv_sp_func_t)(void *user, float *spectra, const b200conv_sp_frame_t *frames_dev,
+                                   const b200conv_sp_frame_t *frames_host, size_t nframes, size_t rank, void *stream);
 
 int     b200conv_sp_create(b200conv_sp_t **out, int device, size_t instances, size_t max_rank);
 void    b200conv_sp_free(b200conv_sp_t *s);
@@ -442,6 +477,8 @@ int     b200conv_sp_set_phase(b200conv_sp_t *s, size_t idx, float phase);
 int     b200conv_sp_bind_complex(b200conv_sp_t *s, size_t idx, const float *table);
 int     b200conv_sp_bind_gain(b200conv_sp_t *s, size_t idx, const float *gain);
 int     b200conv_sp_unbind(b200conv_sp_t *s, size_t idx);
+int     b200conv_sp_set_function(b200conv_sp_t *s, b200conv_sp_func_t fn, void *user);
+int     b200conv_sp_bind_function(b200conv_sp_t *s, size_t idx);
 int     b200conv_sp_process_device(b200conv_sp_t *s, float *dst, size_t dst_stride, const float *src,
                                    size_t src_stride, size_t count, void *stream);
 int     b200conv_sp_process_planar(b200conv_sp_t *s, float *dst, const float *src, size_t stride, size_t count);

@@ -45,6 +45,23 @@ class Stats(ctypes.Structure):
                                                "mac_launches", "mac_algo_bytes", "mac_stream_bytes")]
 
 
+class SpFrame(ctypes.Structure):
+    """b200conv_sp_frame_t: one frame handed to a SpectralProcessorBatch's spectral function."""
+    _fields_ = [("instance", ctypes.c_uint32), ("pos", ctypes.c_uint32)]
+
+
+# b200conv_sp_func_t(user, spectra, frames_dev, frames_host, nframes, rank, stream)
+SP_FUNC = ctypes.CFUNCTYPE(None, _VP, _VP, _VP, _VP, _SZ, _SZ, _VP)
+
+
+class _DeviceArray:
+    """A device buffer of the library seen through ``__cuda_array_interface__`` (no copy, no owner)."""
+
+    def __init__(self, ptr, shape, typestr):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False),
+                                         "version": 2}
+
+
 class B200ConvError(RuntimeError):
     def __init__(self, code, text):
         super().__init__("b200conv error %d: %s" % (code, text))
@@ -133,6 +150,8 @@ _SIGNATURES = {
     "b200conv_sp_bind_complex": (ctypes.c_int, [_VP, _SZ, _FP]),
     "b200conv_sp_bind_gain": (ctypes.c_int, [_VP, _SZ, _FP]),
     "b200conv_sp_unbind": (ctypes.c_int, [_VP, _SZ]),
+    "b200conv_sp_set_function": (ctypes.c_int, [_VP, SP_FUNC, _VP]),
+    "b200conv_sp_bind_function": (ctypes.c_int, [_VP, _SZ]),
     "b200conv_sp_process_device": (ctypes.c_int, [_VP, _VP, _SZ, _VP, _SZ, _SZ, _VP]),
     "b200conv_sp_process_planar": (ctypes.c_int, [_VP, _VP, _VP, _SZ, _SZ]),
     "b200conv_sp_reset": (ctypes.c_int, [_VP]),
@@ -559,11 +578,14 @@ class EqualizerBatch:
 
 class SpectralProcessorBatch:
     """``instances`` x ``lsp::dspu::SpectralProcessor`` on one GPU (``b200conv_sp_*``): same method
-    names and meaning as the reference class; the host callback of the reference is replaced by a
-    per-instance spectral table (``bind_complex`` / ``bind_gain``)."""
+    names and meaning as the reference class.  The spectral operation of an instance is a table
+    (``bind_complex`` / ``bind_gain``) or the object's spectral function (``set_function`` +
+    ``bind_function``), which runs on the device between the forward and inverse transforms."""
 
     def __init__(self, instances, max_rank, device=-1):
         self._h = _VP()
+        self._cfn = None            # the SP_FUNC object the library holds: kept alive while it is set
+        self._exc = None            # an exception raised by the spectral function, re-raised by the call
         _check(lib().b200conv_sp_create(ctypes.byref(self._h), device, instances, max_rank))
         self.instances = instances
 
@@ -608,6 +630,46 @@ class SpectralProcessorBatch:
     def unbind(self, idx):
         _check(lib().b200conv_sp_unbind(self._h, idx))
 
+    def set_function(self, fn):
+        """The object's spectral function, ``fn(spectra, instances, positions, rank)``, or None.
+
+        ``spectra`` is a ``torch.complex64`` CUDA tensor ``[n, 2**rank]`` over the library's buffer
+        (no copy): frame ``f`` holds the packed complex spectrum the reference hands to its callback,
+        and ``fn`` edits it in place.  ``instances`` and ``positions`` are int64 CUDA tensors ``[n]``:
+        the instance of each frame and the sample of the caller's process call at which the reference
+        calls its function.  Frames are ordered by instance, then time.  ``fn`` runs on the calling
+        thread inside ``process`` / ``process_device``, within ``torch.cuda.stream`` of the call's
+        stream, so plain torch operations are ordered with the transforms; the tensors are valid
+        until it returns.  An exception raised by ``fn`` is re-raised when the process call returns;
+        the call itself completes with whatever the spectra then hold."""
+        if fn is None:
+            _check(lib().b200conv_sp_set_function(self._h, SP_FUNC(), None))
+            self._cfn = None
+            return
+
+        def trampoline(user, spectra, frames_dev, frames_host, nframes, rank, stream):
+            try:
+                import torch
+                with torch.cuda.stream(torch.cuda.ExternalStream(stream)):
+                    X = torch.as_tensor(_DeviceArray(spectra, (nframes, 1 << rank), "<c8"), device="cuda")
+                    frames = torch.as_tensor(_DeviceArray(frames_dev, (nframes, 2), "<i4"), device="cuda").long()
+                    fn(X, frames[:, 0], frames[:, 1] & 0xFFFFFFFF, rank)
+            except BaseException as e:          # noqa: BLE001 -- nothing may unwind through the C frame
+                if self._exc is None:
+                    self._exc = e
+
+        cfn = SP_FUNC(trampoline)
+        _check(lib().b200conv_sp_set_function(self._h, cfn, None))
+        self._cfn = cfn
+
+    def bind_function(self, idx):
+        _check(lib().b200conv_sp_bind_function(self._h, idx))
+
+    def _reraise(self):
+        e, self._exc = self._exc, None
+        if e is not None:
+            raise e
+
     def reset(self):
         _check(lib().b200conv_sp_reset(self._h))
 
@@ -617,11 +679,15 @@ class SpectralProcessorBatch:
         if src.ndim != 2 or src.shape[0] != self.instances:
             raise ValueError("expected [instances][samples]")
         out = np.empty_like(src)
-        _check(lib().b200conv_sp_process_planar(self._h, out.ctypes.data, src.ctypes.data, src.shape[1], src.shape[1]))
+        rc = lib().b200conv_sp_process_planar(self._h, out.ctypes.data, src.ctypes.data, src.shape[1], src.shape[1])
+        self._reraise()
+        _check(rc)
         return out
 
     def process_device(self, dst_ptr, dst_stride, src_ptr, src_stride, samples, stream=None):
-        _check(lib().b200conv_sp_process_device(self._h, dst_ptr, dst_stride, src_ptr, src_stride, samples, stream))
+        rc = lib().b200conv_sp_process_device(self._h, dst_ptr, dst_stride, src_ptr, src_stride, samples, stream)
+        self._reraise()
+        _check(rc)
 
     def sync(self):
         _check(lib().b200conv_sp_sync(self._h))
